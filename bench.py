@@ -2,13 +2,17 @@
 """bench.py -- throughput of the LiDAR pillar-encode (+ early-fusion) hot path.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload lidar|fusion]
+                    [--dump-outputs DIR]
 
 A step is one pass of the hot path over one batch of synthetic tiles (BASELINE.json configs[1]: Pix2Poly
 LiDAR-only, 224 px tiles, 100k points per tile, batch 16 per GPU).  Under torchrun (N > 1) every rank encodes its
 own batch (tiles are independent units: no collective on the data path, weak scaling), the step time is the MAX
 over ranks and `value` is the whole-job tiles/s.  One JSON line is printed by rank 0.
 
-  value         device-timed (CUDA events), inputs resident in HBM, rotating over input/output sets larger than L2
+  value         device-timed (CUDA events) over exactly K steps issued right after W warm-up steps (from the completion
+                of the last warm-up step to that of the last timed step), inputs resident in HBM, rotating over
+                input/output sets larger than L2
+  sustained     the same loop held for >= --min-seconds (clocks sampled inside)
   e2e           same metric through the public module API with HOST pinned inputs: H2D copy of the step's points +
                 offsets and a D2H read of the step's result checksum inside the timed region
   roofline      the dominant kernel (PFN tensor-core kernel): algorithmic FLOPs / its CUDA-event duration
@@ -46,7 +50,8 @@ C_FEAT = 384
 def parse():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=200)
+    ap.add_argument("--steps", type=int, default=None,
+                    help="timed steps `value` is taken from (default 20000, ~1 s at B = 16; 200 for --impl reference)")
     ap.add_argument("--warmup", type=int, default=20)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--workload", default="lidar", choices=["lidar", "fusion", "fusion_layer"],
@@ -62,8 +67,18 @@ def parse():
     ap.add_argument("--no-graph", action="store_true", help="launch through the C ABI every step instead of CUDA graphs")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-sub-results", action="store_true", help="skip the secondary configurations (tf32, fusion, density points)")
-    ap.add_argument("--min-seconds", type=float, default=2.0, help="length of the sustained timed region `value` is taken from")
-    return ap.parse_args()
+    ap.add_argument("--min-seconds", type=float, default=2.0, help="length of the sustained timed region (and bound of the e2e ones)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last timed step computed as DIR/<name>.npy (float32, rank 0; "
+                         "a seeded sample of the tiles when the output exceeds 64 MB)")
+    args = ap.parse_args()
+    if args.steps is None:
+        args.steps = 20_000 if args.impl == "ours" else 200
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
+    return args
 
 
 def algorithmic_bytes_per_tile(n_points, workload):
@@ -352,7 +367,8 @@ class Workload:
         self.dev_x = [torch.nested.nested_tensor_from_jagged(v, self.dev_offs) for v in self.dev_vals]
         self.pinned_img = self.dev_img = None
         if self.fusion is not None:
-            imgs = [torch.rand(B, 3, 224, 224) for _ in range(min(sets, 8))]
+            imgs = [torch.rand(B, 3, 224, 224, generator=torch.Generator().manual_seed(1000 * (1 + rank) + s))
+                    for s in range(min(sets, 8))]
             self.pinned_img = [p.pin_memory() for p in imgs] if keep_host else None
             self.dev_img = [imgs[s % len(imgs)].to(dev) for s in range(sets)]
             if workload == "fusion_layer":
@@ -401,14 +417,21 @@ class Workload:
         # voxelize + PFN (+ patch embed (+ fusion convolution)); the counter memset is not a kernel
         return 2 if self.fusion is None else (4 if self.workload == "fusion_layer" else 3)
 
-    def time_steps(self, steps, first=0, single=False):
-        """Device time (ms) of `steps` steps issued back to back: the start event precedes the first step on every lane, the
-        end event follows the last step of every lane."""
+    def time_steps(self, steps, first=0, single=False, warmup=0):
+        """Device time (ms) of steps first .. first + steps - 1 issued back to back; the end event follows the last step of
+        every lane.  Without warm-up the start event precedes the first step on every lane.  With `warmup` steps (first -
+        warmup .. first - 1) issued right before them, it follows the last warm-up step on its stream: the window holds
+        `steps` step completions of a full pipeline, whose fill stays in the warm-up."""
         cur = torch.cuda.current_stream(self.dev)
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-        e0.record(cur)
-        for st in self.streams:
-            st.wait_event(e0)
+        if warmup:
+            for i in range(first - warmup, first):
+                self.run_step(i, single)
+            e0.record(self.streams[0 if single else (first - 1) % self.sets % self.lanes])
+        else:
+            e0.record(cur)
+            for st in self.streams:
+                st.wait_event(e0)
         for i in range(steps):
             self.run_step(first + i, single)
         for st in self.streams:
@@ -424,6 +447,25 @@ class Workload:
             total_ms += self.time_steps(chunk, total_steps, single)
             total_steps += chunk
         return total_steps, total_ms
+
+
+DUMP_LIMIT = 64 << 20
+
+
+def dump_outputs(w, i, directory):
+    """Write what step i (completed) handed its caller as `directory`/<name>.npy, fp32: the tokens (B, ny*nx, C) of the
+    lidar and fusion_layer workloads, the concatenated features (B, 2C, ny, nx) of the fusion workload.  Above
+    DUMP_LIMIT bytes a fixed, seeded sample of the tiles is written (ascending tile order).  Returns a description."""
+    out = w.outs[i % w.sets].cpu().numpy()
+    name = "features" if w.workload == "fusion" else "tokens"
+    tiles = np.arange(out.shape[0])
+    if out.nbytes > DUMP_LIMIT:
+        keep = max(1, DUMP_LIMIT // (out.nbytes // out.shape[0]))
+        tiles = np.sort(np.random.default_rng(0).choice(out.shape[0], keep, replace=False))
+    os.makedirs(directory, exist_ok=True)
+    np.save(os.path.join(directory, name + ".npy"), np.ascontiguousarray(out[tiles], dtype=np.float32))
+    return {"dir": directory, "step": i, "files": {name: list(out[tiles].shape)},
+            "tiles": "all" if len(tiles) == out.shape[0] else tiles.tolist()}
 
 
 def conv_roofline(w, peaks):
@@ -545,19 +587,18 @@ def main():
             dist.barrier()
         torch.cuda.synchronize()
 
-    # ---- timed region 1 (the contract's): device time of exactly K steps, max over ranks ---------------------------
-    for i in range(args.warmup):
-        W.run_step(i)
+    # ---- the timed region: device time of exactly K steps right after W warm-up steps, max over ranks ----------------
     barrier()
-    e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-    ms_region1 = W.time_steps(args.steps, first=args.warmup)
+    ms_region = W.time_steps(args.steps, first=args.warmup, warmup=args.warmup)
     barrier()
-    ms = torch.tensor([ms_region1], device=dev)
+    ms = torch.tensor([ms_region], device=dev)
     if world > 1:
         dist.all_reduce(ms, op=dist.ReduceOp.MAX)
     ms_k = float(ms.item())
-    # ---- timed region 2: the same loop held for >= --min-seconds (sustained clocks / power), clocks sampled inside ----
-    # `value` comes from this region: a burst of K steps of ~50 us says nothing about a power-limited serving loop.
+    ms_per_step = ms_k / args.steps
+    value = B * world / (ms_per_step * 1e-3)
+    dumped = dump_outputs(W, args.warmup + args.steps - 1, args.dump_outputs) if (args.dump_outputs and rank == 0) else None
+    # ---- the same loop held for >= --min-seconds (sustained clocks / power), clocks sampled inside ---------------------
     sampler = ClockSampler(local_rank)
     barrier()
     sampler.start()
@@ -567,8 +608,10 @@ def main():
     t = torch.tensor([sus_ms / sus_steps], device=dev)
     if world > 1:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
-    ms_per_step = float(t.item())
-    value = B * world / (ms_per_step * 1e-3)
+    sustained = {"steps": sus_steps, "seconds": sus_ms * 1e-3, "ms_per_step": float(t.item()),
+                 "value": B * world / (float(t.item()) * 1e-3), "unit": UNIT,
+                 "what": f"the same step loop held for >= {args.min_seconds} s (max over ranks of the per-step time; clocks "
+                         "sampled inside): the power-limited serving loop"}
     one_steps, one_ms = W.time_for(min(0.5, args.min_seconds), single=True)
     t1 = torch.tensor([one_ms / one_steps], device=dev)
     if world > 1:
@@ -576,13 +619,12 @@ def main():
     one_in_flight = {"ms_per_step": float(t1.item()), "value": B * world / (float(t1.item()) * 1e-3), "unit": UNIT, "steps": one_steps,
                      "what": "the same graphs replayed on ONE stream: a step starts when the previous one has ended (the latency-"
                              "oriented number; `value` keeps `in_flight` batches in flight on as many streams / workspaces)"}
-    burst = {"steps": args.steps, "ms_per_step": ms_k / args.steps, "value": B * world * args.steps / (ms_k * 1e-3), "unit": UNIT,
-             "what": "exactly --steps steps between two events (short: boost clocks, no power limit)"}
 
     # ---- end to end through the module API with host buffers ------------------------------------------------------
     # Every step copies its inputs from pinned host memory and reads its result back; the copy of step i + 1 runs on a
     # side stream while step i computes (two device input buffers), as a serving loop would prefetch its next batch.
     nbuf = 2
+    e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     d_vals = [torch.empty_like(W.dev_vals[0]) for _ in range(nbuf)]
     d_offs = [torch.empty_like(W.dev_offs) for _ in range(nbuf)]
     d_img = [torch.empty_like(W.dev_img[0]) for _ in range(nbuf)] if fusion is not None else None
@@ -757,9 +799,10 @@ def main():
     bytes_tile = algorithmic_bytes_per_tile(N, args.workload)
     per_gpu_gbs = bytes_tile * (value / world) / 1e9
     hbm = {"bound": "hbm", "achieved": per_gpu_gbs, "peak": hbm_peak, "unit": "GB/s", "frac": per_gpu_gbs / hbm_peak,
-           "bytes_per_tile": bytes_tile, "peak_source": which, "scope": "whole path, per GPU, sustained region",
+           "bytes_per_tile": bytes_tile, "peak_source": which, "scope": "whole path, per GPU, timed region (`value`)",
            "whole_path_tflops": flops * (value / world / B) / 1e12,
-           "whole_path_frac_of_sustained_tensor_peak": flops * (value / world / B) / 1e12 / (bf16_sus / (2.0 if half else 1.0))}
+           # the sustained loop's rate against the sustained peak
+           "whole_path_frac_of_sustained_tensor_peak": flops * (sustained["value"] / world / B) / 1e12 / (bf16_sus / (2.0 if half else 1.0))}
 
     # ---- secondary configurations, so that the driver's line carries them (BASELINE configs 2-5) -----------------------
     subs = []
@@ -803,9 +846,10 @@ def main():
             "ms_per_step": ms_per_step, "higher_is_better": True, "scaling": "weak", "vs_baseline": None,
             "dtype": {"fp32": "f32", "tf32": "tf32", "bf16": "bf16", "fp16": "f16 operands, f32 accumulate, f32 in/out"}[args.precision], "data": "synthetic",
             "config": workload_config(args), "mpoints_per_s": value * N / 1e6,
-            "timed_region": {"steps_timed": sus_steps, "seconds": sus_ms * 1e-3, "what": f"`value` / `ms_per_step`: the step loop held for >= {args.min_seconds} s "
-                             "(max over ranks of the per-step time); `burst` is the contract's exactly-K-steps region"},
-            "burst": burst, "one_batch_in_flight": one_in_flight,
+            "timed_region": {"steps_timed": args.steps, "warmup_steps": args.warmup, "seconds": ms_k * 1e-3,
+                             "what": "`value` / `ms_per_step`: exactly --steps steps issued right after --warmup warm-up steps, "
+                                     "from the completion of the last warm-up step to that of the last timed step (max over ranks)"},
+            "sustained": sustained, "one_batch_in_flight": one_in_flight, "dump_outputs": dumped,
             "e2e": e2e, "gpu_launches": W.launches_per_step * (args.steps + sus_steps), "launch_mode": "cuda_graph" if W.graphs else "c_abi_per_step",
             "roofline": roofline, "hbm_roofline": hbm, "stage_ms": stage_ms, "sub_results": subs, "cpu_baseline": cpu_baseline, "clocks": clocks,
         }

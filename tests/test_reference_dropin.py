@@ -1,24 +1,33 @@
-"""Drop-in check against the REFERENCE's own files (CPU; runs where /root/reference exists, skipped elsewhere).
+"""The module as the PixelsPointsPolygons project's encoders use it (CPU, plus the shapes of the real forward on the GPU).
 
-The reference's encoder classes are imported unmodified from /root/reference with the single swap INTEGRATION.md
-describes -- `pixelspointspolygons.models.pointpillars.pointpillars_o3d` provided by this package instead of the Open3D
-subclass -- and a stub `timm` (the ViT blocks are out of scope).  cfg comes from the reference's own YAML through PyYAML.
-What is checked here without a GPU: the reference constructors accept our module (same signature, cfg fields, kwargs),
-it lands where the reference puts it (`vit.patch_embed`, `lidar_embed`), the reference's `forward` drives it with the
-arguments we implement (`x_lidar`, `return_flattened`), shapes flow through the reference's own post-processing, and a
-checkpoint saved from the reference-shaped model loads with the reference's key names.  (The arithmetic of the module is
-covered by the -m gpu parity tests; this file pins the boundary.)"""
+On every checkout the module is checked against what the project expects of it, recorded from its source in
+tests/golden/reference_dropin.json: the constructor call and the cfg fields it reads (its encoder YAMLs), the Open3D-ML
+kwargs the constructor derives, the state-dict key names and shapes its checkpoints store, the `forward` arguments its
+encoders pass and the shapes they consume.
+
+Where the environment variable P3P_REFERENCE_DIR names a checkout of the project, the same tests also import its
+encoder classes unmodified with the single swap INTEGRATION.md describes -- `pixelspointspolygons.models.pointpillars.
+pointpillars_o3d` provided by this package instead of the Open3D subclass -- and a stub `timm` (the ViT blocks are out of
+scope), with cfg from the project's own YAML through PyYAML: the reference constructors accept our module, it lands where
+the reference puts it (`vit.patch_embed`, `lidar_embed`), the reference's `forward` drives it with the arguments we
+implement, shapes flow through the reference's own post-processing, and the reference's key names load.  (The
+arithmetic of the module is covered by the -m gpu parity tests; this file pins the boundary.)"""
 import importlib.util
+import inspect
+import json
 import os
 import sys
 import types
 
+import numpy as np
 import pytest
 import torch
 import torch.nn as nn
 
-REF = "/root/reference"
-pytestmark = pytest.mark.skipif(not os.path.isdir(os.path.join(REF, "pixelspointspolygons")), reason="reference tree not present")
+REF = os.environ.get("P3P_REFERENCE_DIR", "")
+LIVE = bool(REF) and os.path.isdir(os.path.join(REF, "pixelspointspolygons"))
+with open(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "reference_dropin.json")) as f:
+    FACTS = json.load(f)
 
 
 class StubViT(nn.Module):
@@ -39,8 +48,7 @@ class StubViT(nn.Module):
         return x + self.pos_embed
 
 
-@pytest.fixture()
-def reference_modules(monkeypatch, tmp_path):
+def load_reference(monkeypatch, tmp_path):
     import pixelspointspolygons_b200 as ours
 
     created = []
@@ -105,11 +113,11 @@ def fake_kernel(monkeypatch, calls):
     monkeypatch.setattr(PointPillarsEncoder, "forward", forward)
 
 
-def test_reference_pointpillars_vit_accepts_the_module(reference_modules, monkeypatch):
+def live_pointpillars_vit(monkeypatch, tmp_path):
     from pixelspointspolygons_b200 import PointPillarsEncoder
     from pixelspointspolygons_b200.config import cfg_from_encoder_yaml
 
-    ppvit, _, created, out_path = reference_modules
+    ppvit, _, created, out_path = load_reference(monkeypatch, tmp_path)
     cfg = cfg_from_encoder_yaml(os.path.join(REF, "config", "encoder", "pointpillars_vit.yaml"), device="cpu", out_path=out_path)
     model = ppvit.PointPillarsViT(cfg, bottleneck=True)
     assert created == ["vit_small_patch8_224.dino"]
@@ -130,11 +138,11 @@ def test_reference_pointpillars_vit_accepts_the_module(reference_modules, monkey
     assert model.vit.seen == (2, 784, 384) and tuple(y.shape) == (2, 784, 256)
 
 
-def test_reference_early_fusion_vit_accepts_the_module(reference_modules, monkeypatch):
+def live_early_fusion_vit(monkeypatch, tmp_path):
     from pixelspointspolygons_b200 import ConvBnRelu3x3, PointPillarsEncoder
     from pixelspointspolygons_b200.config import cfg_from_encoder_yaml
 
-    _, efvit, _, out_path = reference_modules
+    _, efvit, _, out_path = load_reference(monkeypatch, tmp_path)
     cfg = cfg_from_encoder_yaml(os.path.join(REF, "config", "encoder", "early_fusion_vit.yaml"), device="cpu", out_path=out_path)
     model = efvit.EarlyFusionViT(cfg)
     assert isinstance(model.lidar_embed, PointPillarsEncoder)
@@ -151,3 +159,83 @@ def test_reference_early_fusion_vit_accepts_the_module(reference_modules, monkey
     y = model(torch.rand(2, 3, 224, 224), x_lidar)
     assert calls and calls[0][1:] == (2, False)  # lidar_embed(x_lidar, return_flattened=False)
     assert tuple(y.shape) == (2, 784, 256)
+
+
+def stored_cfg(device="cpu"):
+    from pixelspointspolygons_b200.config import AttrDict
+
+    enc = {k: v for k, v in FACTS["encoder_cfg"].items() if k != "source"}
+    return AttrDict.wrap(dict(host=dict(device=device), run_type=dict(logging="WARNING"),
+                              experiment=dict(encoder=enc, lidar_dropout=None)))
+
+
+def stored_encoder(device="cpu"):
+    from pixelspointspolygons_b200 import PointPillarsEncoder
+
+    ctor = FACTS["constructor"]
+    return PointPillarsEncoder(stored_cfg(device), voxel_encoder=ctor["voxel_encoder"], scatter=ctor["scatter"],
+                               local_rank=ctor["local_rank"])
+
+
+def keys_and_shapes(module):
+    """name -> shape (a checkpoint loads by name: the order of the keys is not part of the format)"""
+    return {k: list(t.shape) for k, t in module.state_dict().items()}
+
+
+def stored(entry):
+    return {k: s for k, s in FACTS[entry]["keys"]}
+
+
+def check_stored_encoder():
+    """The constructor call of the reference's encoders, the kwargs it derives, its checkpoint keys, its forward signature."""
+    from pixelspointspolygons_b200 import PointPillarsEncoder
+
+    enc = stored_encoder()
+    for name, value in FACTS["constructed"].items():
+        if name != "source":
+            assert getattr(enc, name) == value, name
+    assert keys_and_shapes(enc) == stored("state_dict")
+    # a checkpoint with the reference's names and shapes loads strictly, and comes back under the same names
+    sd = {k: torch.zeros(s, dtype=torch.long) if k.endswith("num_batches_tracked") else torch.rand(s)
+          for k, s in stored("state_dict").items()}
+    enc.load_state_dict(sd, strict=True)
+    assert all(torch.equal(enc.state_dict()[k], v) for k, v in sd.items())
+    params = inspect.signature(PointPillarsEncoder.forward).parameters
+    assert list(params)[1:3] == ["x_lidar", "return_flattened"] and params["return_flattened"].default is True
+
+
+def test_reference_pointpillars_vit_accepts_the_module(monkeypatch, tmp_path):
+    check_stored_encoder()
+    if LIVE:
+        live_pointpillars_vit(monkeypatch, tmp_path)
+
+
+def test_reference_early_fusion_vit_accepts_the_module(monkeypatch, tmp_path):
+    from pixelspointspolygons_b200 import ConvBnRelu3x3
+    from pixelspointspolygons_b200.fusion import EarlyFusionFrontEnd
+
+    check_stored_encoder()
+    fe = EarlyFusionFrontEnd(stored_cfg())
+    assert keys_and_shapes(fe.fusion_layer) == stored("fusion_layer_state_dict")
+    assert keys_and_shapes(fe.image_embed) == stored("image_embed_state_dict")
+    assert keys_and_shapes(fe.lidar_embed) == stored("state_dict")
+    ours = ConvBnRelu3x3(768, 384)
+    sd = {k: torch.zeros(s, dtype=torch.long) if k.endswith("num_batches_tracked") else torch.rand(s)
+          for k, s in stored("fusion_layer_state_dict").items()}
+    ours.load_state_dict(sd, strict=True)
+    if LIVE:
+        live_early_fusion_vit(monkeypatch, tmp_path)
+
+
+@pytest.mark.gpu
+@pytest.mark.parametrize("encoder", ["pointpillars_vit", "early_fusion_vit"])
+def test_forward_hands_the_reference_the_shapes_it_consumes(cuda_device, encoder):
+    from tools.synth import synth_tile
+
+    want = FACTS["forward"][encoder]
+    enc = stored_encoder(str(cuda_device)).to(cuda_device).eval()
+    x = torch.nested.nested_tensor([torch.from_numpy(synth_tile(n, 70 + n)) for n in (50, 7)], layout=torch.jagged).to(cuda_device)
+    with torch.no_grad():
+        y = enc(x, return_flattened=want["return_flattened"])
+    assert list(y.shape) == [2] + want["shape_per_tile"] and y.dtype == torch.float32 and y.is_cuda
+    assert np.isfinite(y.cpu().numpy()).all()
