@@ -272,6 +272,20 @@ int p3p_conv3x3(const void* x, int32_t num_tiles, int32_t height, int32_t width,
                 int32_t out_channels, int32_t precision, int32_t relu, float* out, int32_t out_layout, int32_t c_total,
                 int32_t c_offset, void* stream);
 
+/*
+ * The early-fusion ViT input in the same launch: p3p_conv3x3 (ReLU on) followed by what timm's
+ * `VisionTransformer._pos_embed` does to the fusion layer's token rows in `EarlyFusionViT.forward`
+ * (early_fusion_vit.py:123-124: `x = self.fusion_layer(x).flatten(2).transpose(1, 2)`, then `vit.forward_features(x)`
+ * with `patch_embed = Identity`; one class token, no register tokens, `no_embed_class = False`):
+ *   out[b, 0, :]       = cls_token + pos_embed[0, :]
+ *   out[b, 1 + pos, :] = ReLU(BatchNorm2d(Conv2d(x)))[b, :, pos] + pos_embed[1 + pos, :]      pos = y W + x
+ * out: (B, 1 + H W, Cout) fp32; cls_token: (Cout) fp32; pos_embed: (1 + H W, Cout) fp32, all on the device.  x, blob,
+ * precision and the error codes as p3p_conv3x3; a null cls_token or pos_embed is P3P_ERR_INVALID_ARGUMENT.
+ */
+int p3p_conv3x3_vit_tokens(const void* x, int32_t num_tiles, int32_t height, int32_t width, int32_t in_channels, const void* blob,
+                           int32_t out_channels, int32_t precision, const float* cls_token, const float* pos_embed, float* out,
+                           void* stream);
+
 /* fp32 NCHW (B, C, H, W) -> 16-bit channels-last (B, H, W, c_total) at channel offset c_offset. */
 int p3p_nchw_to_nhwc16(const float* x, int32_t num_tiles, int32_t channels, int32_t height, int32_t width, int32_t precision,
                        void* out, int32_t c_total, int32_t c_offset, void* stream);

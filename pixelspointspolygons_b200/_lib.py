@@ -15,7 +15,7 @@ P3P_GRID_DROP_OVERFLOW = 1
 EXPORTED = [
     "p3p_last_error", "p3p_version", "p3p_workspace_bytes", "p3p_pfn_blob_bytes", "p3p_pfn_prepare",
     "p3p_voxelize", "p3p_pillar_features", "p3p_encode", "p3p_encode_tokens", "p3p_patch_embed", "p3p_las_to_pixels",
-    "p3p_profile_begin", "p3p_profile_end", "p3p_conv3x3_blob_bytes", "p3p_conv3x3_prepare", "p3p_conv3x3",
+    "p3p_profile_begin", "p3p_profile_end", "p3p_conv3x3_blob_bytes", "p3p_conv3x3_prepare", "p3p_conv3x3", "p3p_conv3x3_vit_tokens",
     "p3p_nchw_to_nhwc16", "p3p_upsample_bilinear_nhwc16", "p3p_las_packed_to_pixels",
     "p3p_patch_embed_blob_bytes", "p3p_patch_embed_prepare", "p3p_patch_embed_prepared",
     "p3p_encode_workspace", "p3p_pfn_train_state_doubles", "p3p_pfn_train_route_bytes", "p3p_pfn_train_stats0",
@@ -111,6 +111,8 @@ def lib():
     l.p3p_conv3x3_prepare.argtypes = [C.POINTER(ConvParams), i32, vp, sz, vp]
     l.p3p_conv3x3.restype = C.c_int
     l.p3p_conv3x3.argtypes = [vp, i32, i32, i32, i32, vp, i32, i32, i32, vp, i32, i32, i32, vp]
+    l.p3p_conv3x3_vit_tokens.restype = C.c_int
+    l.p3p_conv3x3_vit_tokens.argtypes = [vp, i32, i32, i32, i32, vp, i32, i32, vp, vp, vp, vp]
     l.p3p_nchw_to_nhwc16.restype = C.c_int
     l.p3p_nchw_to_nhwc16.argtypes = [vp, i32, i32, i32, i32, i32, vp, i32, i32, vp]
     l.p3p_upsample_bilinear_nhwc16.restype = C.c_int

@@ -450,6 +450,18 @@ int p3p_conv3x3(const void* x, int32_t num_tiles, int32_t height, int32_t width,
                           static_cast<cudaStream_t>(stream));
 }
 
+int p3p_conv3x3_vit_tokens(const void* x, int32_t num_tiles, int32_t height, int32_t width, int32_t in_channels, const void* blob,
+                           int32_t out_channels, int32_t precision, const float* cls_token, const float* pos_embed, float* out,
+                           void* stream) {
+    if (num_tiles < 0 || height < 1 || width < 1 || in_channels < 1 || out_channels < 1) return fail(P3P_ERR_INVALID_ARGUMENT, "bad sizes");
+    if (!cls_token || !pos_embed) return fail(P3P_ERR_INVALID_ARGUMENT, "cls_token or pos_embed is null");
+    if (num_tiles == 0) return P3P_OK;
+    if (!x || !blob || !out) return fail(P3P_ERR_INVALID_ARGUMENT, "null x, blob or out");
+    if (!aligned16(x) || !aligned16(blob) || !aligned16(out)) return fail(P3P_ERR_INVALID_ARGUMENT, "misaligned pointer");
+    return launch_conv3x3_vit_tokens(x, num_tiles, height, width, in_channels, blob, out_channels, precision, cls_token, pos_embed, out,
+                                     static_cast<cudaStream_t>(stream));
+}
+
 int p3p_nchw_to_nhwc16(const float* x, int32_t num_tiles, int32_t channels, int32_t height, int32_t width, int32_t precision,
                        void* out, int32_t c_total, int32_t c_offset, void* stream) {
     if (num_tiles < 0 || channels < 1 || height < 1 || width < 1) return fail(P3P_ERR_INVALID_ARGUMENT, "bad sizes");

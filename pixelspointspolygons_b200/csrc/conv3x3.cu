@@ -19,6 +19,13 @@
 // (64, 128) of Wp per channel tile.  Warp 0 produces (TMA + mbarrier expect_tx), warps 1-3 issue tcgen05.mma (one channel tile each) and
 // release the stages with tcgen05.commit, warps 4-7 drain TMEM: + shift, ReLU, store as token rows (B, H W, Cout) -- the
 // `.flatten(2).transpose(1, 2)` of the reference is the store address -- or NCHW.
+//
+// ViT-token epilogue (template flag kVitTokens; the NLC / NCHW instantiation is compiled without it): the output is the
+// ViT's input sequence (B, 1 + H W, Cout), what timm's `_pos_embed` makes of the token rows (early_fusion_vit.py:123-124):
+// position pos of image b goes to row b (1 + H W) + 1 + pos as relu(acc + shift) + pos_embed[1 + pos] -- BN, ReLU, then the
+// fp32 add, the reference's order -- and the epilogue warps of the CTA holding strip 0 of an image write its row 0,
+// cls_token + pos_embed[0], while the MMAs run.  pos_embed is read as the rows are stored: 32 consecutive channels of one
+// position per warp access.
 #include <cuda.h>
 #include <cuda_fp16.h>
 
@@ -49,6 +56,8 @@ struct ConvArgs {
     float* out;
     int out_layout;        // P3P_LAYOUT_NLC: (B, H W, c_total) rows at c_offset; P3P_LAYOUT_NCHW: (B, c_total, H, W)
     int c_total, c_offset;
+    const float* cls_token;  // (Cout)                  ViT-token epilogue only
+    const float* pos_embed;  // ((1 + H W), Cout)       ViT-token epilogue only
 };
 
 __device__ __forceinline__ void mbar_expect_tx(uint64_t* bar, uint32_t bytes) {
@@ -76,6 +85,7 @@ __device__ __forceinline__ void tmem_ld16(uint32_t taddr, float (&v)[16]) {
         : "memory");
 }
 
+template <bool kVitTokens>
 __global__ void __launch_bounds__(kConvThreads, 1)
 conv3x3_tc_kernel(const __grid_constant__ CUtensorMap tm_x, const __grid_constant__ CUtensorMap tm_w, ConvArgs a) {
     extern __shared__ __align__(1024) unsigned char smem_dyn[];  // no static shared memory below: the block starts at offset 0
@@ -162,6 +172,13 @@ conv3x3_tc_kernel(const __grid_constant__ CUtensorMap tm_x, const __grid_constan
     } else {
         // =========================== epilogue: thread = output channel (TMEM lane), columns = positions ===================
         const int quad = warp & 3;
+        if constexpr (kVitTokens) {
+            // the class-token row of this image, while the MMAs run
+            if (strip == 0) {
+                float* row0 = a.out + (int64_t)b * (a.H * a.W + 1) * a.Cout;
+                for (int c = tid - 4 * 32; c < a.Cout; c += 4 * 32) row0[c] = a.cls_token[c] + a.pos_embed[c];
+            }
+        }
         mbar_wait(acc_full, 0);
         tc_fence_after();
         const int HW = a.H * a.W;
@@ -179,7 +196,18 @@ conv3x3_tc_kernel(const __grid_constant__ CUtensorMap tm_x, const __grid_constan
                     if (a.relu) v[i] = fmaxf(v[i], 0.f);
                 }
                 if (co < a.Cout) {
-                    if (a.out_layout == P3P_LAYOUT_NLC) {
+                    if constexpr (kVitTokens) {
+                        // token row 1 + pos of image b, + pos_embed[1 + pos]: the same coalesced pattern on both sides
+                        const int64_t r0 = 1 + pos0 + j0;
+                        float* dst = a.out + ((int64_t)b * (HW + 1) + r0) * a.Cout + co;
+                        const float* pe = a.pos_embed + r0 * a.Cout + co;
+                        float p[16];
+#pragma unroll
+                        for (int i = 0; i < 16; ++i) p[i] = pos0 + j0 + i < HW ? __ldg(pe + (int64_t)i * a.Cout) : 0.f;
+#pragma unroll
+                        for (int i = 0; i < 16; ++i)
+                            if (pos0 + j0 + i < HW) dst[(int64_t)i * a.Cout] = v[i] + p[i];
+                    } else if (a.out_layout == P3P_LAYOUT_NLC) {
                         // token rows: a warp writes 32 consecutive channels of one position per store
                         float* dst = a.out + ((int64_t)b * HW + pos0 + j0) * a.c_total + a.c_offset + co;
 #pragma unroll
@@ -340,8 +368,11 @@ int launch_upsample_bilinear_nhwc16(const float* x, int B, int h, int w, int C, 
     return P3P_OK;
 }
 
-int launch_conv3x3(const void* x, int B, int H, int W, int Cin, const void* blob, int Cout, int precision, int relu, float* out,
-                   int out_layout, int c_total, int c_offset, cudaStream_t st) {
+namespace {
+
+// cls_token / pos_embed non-null: the ViT-token epilogue (out: (B, 1 + H W, Cout); out_layout, c_total, c_offset unused)
+int launch_conv3x3_any(const void* x, int B, int H, int W, int Cin, const void* blob, int Cout, int precision, int relu, float* out,
+                       int out_layout, int c_total, int c_offset, const float* cls_token, const float* pos_embed, cudaStream_t st) {
     if (B <= 0) return P3P_OK;
     if (precision != P3P_PRECISION_BF16 && precision != P3P_PRECISION_FP16)
         return fail(P3P_ERR_UNSUPPORTED, "conv3x3 runs on 16-bit operands (precision bf16 or fp16), got %d", precision);
@@ -371,6 +402,7 @@ int launch_conv3x3(const void* x, int B, int H, int W, int Cin, const void* blob
     const int cout_pad = co_tiles * 128;
     a.shift = reinterpret_cast<const float*>(static_cast<const char*>(blob) + (size_t)cout_pad * 9 * Cin * 2);
     a.out = out; a.out_layout = out_layout; a.c_total = c_total; a.c_offset = c_offset;
+    a.cls_token = cls_token; a.pos_embed = pos_embed;
 
     CUtensorMap tm_x, tm_w;
     const CUtensorMapDataType dt = precision == P3P_PRECISION_BF16 ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT16;
@@ -393,7 +425,8 @@ int launch_conv3x3(const void* x, int B, int H, int W, int Cin, const void* blob
         if (r != CUDA_SUCCESS) return fail(P3P_ERR_CUDA, "cuTensorMapEncodeTiled (weights) failed: %d", (int)r);
     }
     const size_t smem = (size_t)a.stages * a.stage_bytes + (2 * 8 + 1) * 8 + 16;
-    P3P_CUDA_CHECK(cudaFuncSetAttribute(conv3x3_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    auto* kernel = pos_embed ? conv3x3_tc_kernel<true> : conv3x3_tc_kernel<false>;
+    P3P_CUDA_CHECK(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     cudaLaunchAttribute attr[1];
     attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
     attr[0].val.programmaticStreamSerializationAllowed = 1;
@@ -404,9 +437,21 @@ int launch_conv3x3(const void* x, int B, int H, int W, int Cin, const void* blob
     cfg.stream = st;
     cfg.attrs = attr;
     cfg.numAttrs = 1;
-    P3P_CUDA_CHECK(cudaLaunchKernelEx(&cfg, conv3x3_tc_kernel, tm_x, tm_w, a));
+    P3P_CUDA_CHECK(cudaLaunchKernelEx(&cfg, kernel, tm_x, tm_w, a));
     P3P_CUDA_CHECK(cudaGetLastError());
     return P3P_OK;
+}
+
+}  // namespace
+
+int launch_conv3x3(const void* x, int B, int H, int W, int Cin, const void* blob, int Cout, int precision, int relu, float* out,
+                   int out_layout, int c_total, int c_offset, cudaStream_t st) {
+    return launch_conv3x3_any(x, B, H, W, Cin, blob, Cout, precision, relu, out, out_layout, c_total, c_offset, nullptr, nullptr, st);
+}
+
+int launch_conv3x3_vit_tokens(const void* x, int B, int H, int W, int Cin, const void* blob, int Cout, int precision,
+                              const float* cls_token, const float* pos_embed, float* out, cudaStream_t st) {
+    return launch_conv3x3_any(x, B, H, W, Cin, blob, Cout, precision, 1, out, P3P_LAYOUT_NLC, Cout, 0, cls_token, pos_embed, st);
 }
 
 }  // namespace p3p

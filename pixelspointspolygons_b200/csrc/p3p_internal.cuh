@@ -196,6 +196,8 @@ size_t conv3x3_blob_bytes(int Cin, int Cout);
 int launch_conv3x3_prepare(const p3p_conv_params* p, int precision, void* blob, cudaStream_t st);
 int launch_conv3x3(const void* x, int B, int H, int W, int Cin, const void* blob, int Cout, int precision, int relu, float* out,
                    int out_layout, int c_total, int c_offset, cudaStream_t st);
+int launch_conv3x3_vit_tokens(const void* x, int B, int H, int W, int Cin, const void* blob, int Cout, int precision,
+                              const float* cls_token, const float* pos_embed, float* out, cudaStream_t st);
 int launch_nchw_to_nhwc16(const float* x, int B, int C, int H, int W, int precision, void* out, int c_total, int c_offset, cudaStream_t st);
 int launch_upsample_bilinear_nhwc16(const float* x, int B, int h, int w, int C, int64_t src_batch_stride, int H, int W, int precision,
                                     void* out, cudaStream_t st);

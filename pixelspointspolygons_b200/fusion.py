@@ -156,6 +156,29 @@ class _Conv3x3Runner:
         _lib.check(rc, "p3p_conv3x3")
         return out
 
+    def run_vit_tokens(self, x16: torch.Tensor, cls_token: torch.Tensor, pos_embed: torch.Tensor, out: torch.Tensor):
+        """x16 as in `run` -> out (B, 1 + H W, Cout) fp32, the ViT input (p3p_conv3x3_vit_tokens): row 0 of every image
+        cls_token + pos_embed[0], row 1 + pos the convolution + BN + ReLU at pos + pos_embed[1 + pos].  cls_token (Cout) and
+        pos_embed ((1 + H W) Cout values) are contiguous float32 on the device of x; the kernel reads them in place."""
+        if x16.dtype != self.operand_dtype or x16.dim() != 4 or x16.shape[3] != self.in_channels or not x16.is_contiguous():
+            raise TypeError(f"x must be a contiguous {self.operand_dtype} tensor (B, H, W, {self.in_channels})")
+        if not x16.is_cuda:
+            raise RuntimeError("the 3x3 convolution kernel runs on CUDA only (sm_100a); x is on " + str(x16.device))
+        B, H, W, _ = x16.shape
+        Cc, rows = self.out_channels, H * W + 1
+        for name, t, n in (("cls_token", cls_token, Cc), ("pos_embed", pos_embed, rows * Cc)):
+            if t.dtype != torch.float32 or not t.is_contiguous() or t.device != x16.device or t.numel() != n:
+                raise ValueError(f"{name} must be a contiguous float32 tensor of {n} elements on the device of x")
+        if out.dtype != torch.float32 or not out.is_contiguous() or out.device != x16.device or out.numel() < B * rows * Cc:
+            raise ValueError("out must be a contiguous float32 tensor of B * (1 + H * W) * Cout elements on the device of x")
+        with torch.cuda.device(x16.device):
+            blob = self.blob(x16.device)
+            rc = _lib.lib().p3p_conv3x3_vit_tokens(x16.data_ptr(), B, H, W, self.in_channels, blob.data_ptr(), Cc,
+                                                   P3P_PRECISION[self.precision], cls_token.data_ptr(), pos_embed.data_ptr(),
+                                                   out.data_ptr(), torch.cuda.current_stream(x16.device).cuda_stream)
+        _lib.check(rc, "p3p_conv3x3_vit_tokens")
+        return out
+
 
 class ConvBnRelu3x3(nn.Sequential):
     """`nn.Sequential(nn.Conv2d(cin, cout, kernel_size=3, padding=1), nn.BatchNorm2d(cout), nn.ReLU(inplace=True))` -- the
@@ -294,25 +317,58 @@ class EarlyFusionFrontEnd(nn.Module):
             side = self._side_streams[(dev, lane)] = torch.cuda.Stream(dev)
         return side
 
-    def forward_tokens(self, x_image, x_lidar, lidar_zero: Optional[bool] = None) -> torch.Tensor:
+    def _vit_params(self, cls_token, pos_embed, device):
+        """cls_token (1, 1, C) / pos_embed (1, 1 + ny nx, C) as contiguous fp32 on `device` -- the parameters themselves
+        when they already are -- or (None, None) when neither is given."""
+        if (cls_token is None) != (pos_embed is None):
+            raise ValueError("cls_token and pos_embed go together: pass both or neither")
+        if cls_token is None:
+            return None, None
+        hw, Cc = self.lidar_embed.ny * self.lidar_embed.nx, self.channels
+        if cls_token.numel() != Cc or pos_embed.numel() != (hw + 1) * Cc:
+            raise ValueError(f"cls_token must hold {Cc} and pos_embed {(hw + 1) * Cc} values")
+        return (cls_token.detach().to(device=device, dtype=torch.float32).contiguous(),
+                pos_embed.detach().to(device=device, dtype=torch.float32).contiguous())
+
+    def forward_tokens(self, x_image, x_lidar, lidar_zero: Optional[bool] = None, *, cls_token: Optional[torch.Tensor] = None,
+                       pos_embed: Optional[torch.Tensor] = None) -> torch.Tensor:
         """`EarlyFusionViT.forward` through `self.fusion_layer(x).flatten(2).transpose(1, 2)` (early_fusion_vit.py:96-123):
         (B, ny nx, C) fp32 tokens, the ViT's input.  Eval mode: the two producers write their halves of ONE 16-bit
         channels-last buffer (B, ny, nx, 2C) -- the reference's fp32 NCHW concat tensor never exists -- and the implicit-GEMM
-        kernel turns it into token rows."""
+        kernel turns it into token rows.
+
+        With `cls_token` (1, 1, C) and `pos_embed` (1, 1 + ny nx, C) -- the ViT's own parameters -- the result is also
+        passed through timm's `_pos_embed` (early_fusion_vit.py:124, `vit.forward_features` with `patch_embed = Identity`;
+        one class token, `no_embed_class = False`): (B, 1 + ny nx, C) fp32, row 0 = cls_token + pos_embed[0], row 1 + cell =
+        token + pos_embed[1 + cell].  Eval mode writes it from the convolution's epilogue (no cat, no add kernel); train mode
+        runs the torch route above followed by `torch.cat` + add, so gradients reach cls_token and pos_embed."""
         if self.training:
+            if (cls_token is None) != (pos_embed is None):
+                raise ValueError("cls_token and pos_embed go together: pass both or neither")
             x = self.forward(x_image, x_lidar)
-            return self.fusion_layer(x).flatten(2).transpose(1, 2)
+            t = self.fusion_layer(x).flatten(2).transpose(1, 2)
+            if cls_token is None:
+                return t
+            B, hw, Cc = t.shape
+            if cls_token.numel() != Cc or pos_embed.numel() != (hw + 1) * Cc:
+                raise ValueError(f"cls_token must hold {Cc} and pos_embed {(hw + 1) * Cc} values")
+            cls = cls_token.to(device=t.device, dtype=torch.float32).reshape(1, 1, Cc).expand(B, -1, -1)
+            return torch.cat((cls, t), dim=1) + pos_embed.to(device=t.device, dtype=torch.float32).reshape(1, hw + 1, Cc)
         dim, le, fl = self.channels, self.lidar_embed, self.fusion_layer
         B, dev = x_image.shape[0], x_image.device
         x16 = torch.empty(B, le.ny, le.nx, 2 * dim, dtype=fl.operand_dtype, device=dev)
-        out = torch.empty(B, le.ny * le.nx, dim, dtype=torch.float32, device=dev)
-        return self.forward_tokens_into(x_image, x_lidar, x16, out, lidar_zero)
+        rows = le.ny * le.nx + (0 if cls_token is None else 1)
+        out = torch.empty(B, rows, dim, dtype=torch.float32, device=dev)
+        return self.forward_tokens_into(x_image, x_lidar, x16, out, lidar_zero, cls_token=cls_token, pos_embed=pos_embed)
 
     def forward_tokens_into(self, x_image, x_lidar, x16: torch.Tensor, out: torch.Tensor, lidar_zero: Optional[bool] = None,
-                            lane: int = 0):
-        """forward_tokens with caller-owned buffers: x16 (B, ny, nx, 2C) 16-bit scratch, out (B, ny nx, C) fp32."""
+                            lane: int = 0, *, cls_token: Optional[torch.Tensor] = None, pos_embed: Optional[torch.Tensor] = None):
+        """forward_tokens with caller-owned buffers: x16 (B, ny, nx, 2C) 16-bit scratch, out (B, ny nx, C) fp32 -- or
+        (B, 1 + ny nx, C) with cls_token / pos_embed, which the kernel reads in place when they are fp32 on the device
+        (otherwise from a converted copy)."""
         dim, le, fl = self.channels, self.lidar_embed, self.fusion_layer
         dev = x_image.device
+        cls, pos = self._vit_params(cls_token, pos_embed, dev)
         lidar_zero = self._dropout_now(dev) if lidar_zero is None else bool(lidar_zero)
         cur = torch.cuda.current_stream(dev)
         side = self._side_stream(dev, lane)
@@ -321,6 +377,8 @@ class EarlyFusionFrontEnd(nn.Module):
             self.image_embed.forward_into(x_image, x16, 2 * dim, 0, layout=P3P_LAYOUT_NLC)
         le.encode_into(x_lidar, x16, P3P_LAYOUT_NLC, c_total=2 * dim, c_offset=dim, lidar_zero=lidar_zero, lane=lane)
         cur.wait_stream(side)
+        if cls is not None:
+            return fl._runner.run_vit_tokens(x16, cls, pos, out)
         return fl.forward_nhwc(x16, out, P3P_LAYOUT_NLC)
 
     def forward(self, x_image, x_lidar):

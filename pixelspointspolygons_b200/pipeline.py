@@ -55,7 +55,14 @@ class Slot:
 
 class HostPipeline:
     """module: a `PointPillarsEncoder` (LiDAR-only; output (B, ny nx, C) token rows) or an `EarlyFusionFrontEnd`
-    (`mode` = "concat": (B, 2C, ny, nx); "tokens": through `fusion_layer`, (B, ny nx, C)), in eval mode on a CUDA device.
+    (`mode` = "concat": (B, 2C, ny, nx); "tokens": through `fusion_layer`, (B, ny nx, C); "vit_tokens": the ViT's input
+    sequence (B, 1 + ny nx, C) with `cls_token` (1, 1, C) and `pos_embed` (1, 1 + ny nx, C), see
+    `EarlyFusionFrontEnd.forward_tokens`), in eval mode on a CUDA device.
+
+    In "vit_tokens" mode the captured graphs read `cls_token` and `pos_embed` where they are in device memory (they must
+    be contiguous float32 on the module's device): an in-place update -- an optimizer step, `load_state_dict`, `.copy_()`
+    -- is seen by the next batch computed, a tensor put in their place (a new `nn.Parameter`, `.to()` elsewhere) is not;
+    build a new pipeline for that.
 
     Use:
         s = pipe.staging()        # the slot to fill next (blocks only if its previous copy is still in flight)
@@ -66,7 +73,8 @@ class HostPipeline:
     """
 
     def __init__(self, module, B: int, total: int, slots: int = 3, mode: str = "tokens", image_hw: Sequence[int] = (224, 224),
-                 host_result=None, z_hi: float = 100.0, variant: str = "dataset"):
+                 host_result=None, z_hi: float = 100.0, variant: str = "dataset", cls_token: Optional[torch.Tensor] = None,
+                 pos_embed: Optional[torch.Tensor] = None):
         if slots < 2:
             raise ValueError("at least two slots (one in compute, one in copy)")
         p = next(module.parameters())
@@ -78,10 +86,20 @@ class HostPipeline:
         self.device = dev = p.device
         self.fusion = not isinstance(module, PointPillarsEncoder)
         self.mode = mode if self.fusion else "lidar"
-        if self.fusion and mode not in ("concat", "tokens"):
-            raise ValueError("mode must be 'concat' or 'tokens'")
+        if self.fusion and mode not in ("concat", "tokens", "vit_tokens"):
+            raise ValueError("mode must be 'concat', 'tokens' or 'vit_tokens'")
         enc = module.lidar_embed if self.fusion else module
         hw, Cc = enc.ny * enc.nx, enc.channels
+        self._cls = self._pos = None
+        if self.mode == "vit_tokens":
+            if cls_token is None or pos_embed is None:
+                raise ValueError("mode 'vit_tokens' needs cls_token and pos_embed")
+            for name, t in (("cls_token", cls_token), ("pos_embed", pos_embed)):
+                if t.dtype != torch.float32 or t.device != dev or not t.is_contiguous():
+                    raise TypeError(f"{name} must be a contiguous float32 tensor on {dev} (the graphs read it in place)")
+            self._cls, self._pos = cls_token, pos_embed
+        elif cls_token is not None or pos_embed is not None:
+            raise ValueError("cls_token / pos_embed belong to mode 'vit_tokens'")
         self._full = host_result == "full"
         self._reduce: Optional[Callable] = host_result if callable(host_result) else None
         if host_result is not None and not (self._full or self._reduce):
@@ -122,6 +140,8 @@ class HostPipeline:
             s.offsets[self.B] = self.total
             if self.mode == "concat":
                 s.out = torch.empty(self.B, 2 * Cc, enc.ny, enc.nx, dtype=torch.float32, device=dev)
+            elif self.mode == "vit_tokens":
+                s.out = torch.empty(self.B, 1 + hw, Cc, dtype=torch.float32, device=dev)
             else:
                 s.out = torch.empty(self.B, hw, Cc, dtype=torch.float32, device=dev)
             if self._full:
@@ -132,7 +152,7 @@ class HostPipeline:
             self._dev.append(devt)
             self._dviews.append(views(devt, None))
         self._x16 = None
-        if self.mode == "tokens":
+        if self.mode in ("tokens", "vit_tokens"):
             self._x16 = torch.empty(self.B, enc.ny, enc.nx, 2 * Cc, dtype=module.fusion_layer.operand_dtype, device=dev)
         # the LAS arithmetic's per-tile constants come from the slot's own arena (set_tiles), not from a fixed table
         self._fe = LasPackedFrontEnd([], self.total, dev, z_hi, variant, B=self.B)
@@ -177,8 +197,10 @@ class HostPipeline:
             m.encode_into(x, s.out, P3P_LAYOUT_NLC)
         elif self.mode == "concat":
             m.forward_into(d["image"], x, s.out, lidar_zero=False)
-        else:
+        elif self.mode == "tokens":
             m.forward_tokens_into(d["image"], x, self._x16, s.out, lidar_zero=False)
+        else:
+            m.forward_tokens_into(d["image"], x, self._x16, s.out, lidar_zero=False, cls_token=self._cls, pos_embed=self._pos)
         if self._reduce is not None:
             r = self._reduce(s.out)
             if s.host_value is None:
