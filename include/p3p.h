@@ -331,7 +331,9 @@ int p3p_encode_workspace(const p3p_grid* grid, int32_t num_tiles, int64_t total_
  * backward: p3p_pfn_backward1 (grad_out, out: (B, ny nx, C) fp32 rows, route as left by the forward) ->
  *           [back1g] -> p3p_pfn_backward2 -> [back0g] -> p3p_pfn_backward3 (gradients of the six parameters, fp32,
  *           this rank's share: DDP averages them as it does for the reference).
- * Covers C <= 512 and max_points <= 512.
+ * Covers every C <= 512 with every max_points <= 512.  Each entry refuses anything else with P3P_ERR_UNSUPPORTED and a
+ * message naming the limit before it launches or writes anything (p3p_pfn_train_state_doubles returns 0 for such a C).
+ * A batch without pillars is valid: zero output, zero gradients, batch mean and variance 0 with rows = 0.
  */
 int64_t p3p_pfn_train_state_doubles(int32_t channels, int64_t* offsets);
 size_t p3p_pfn_train_route_bytes(const p3p_grid* grid, int32_t num_tiles, int32_t channels);

@@ -33,6 +33,20 @@ int device_sm_count() {
     return sms;
 }
 
+size_t device_smem_optin() {
+    static size_t bytes = 0;
+    if (bytes == 0) {
+        int dev = 0, n = 0;
+        if (cudaGetDevice(&dev) == cudaSuccess &&
+            cudaDeviceGetAttribute(&n, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev) == cudaSuccess && n > 0)
+            bytes = (size_t)n;
+        else
+            bytes = 227 * 1024;  // sm_100 (the only target of this library); keeps the shape checks usable without a GPU
+        (void)cudaGetLastError();
+    }
+    return bytes;
+}
+
 // Same fp32 operation sequence as Open3D VoxelizeCPU / PointPillarsVoxelization (SURVEY A.1, A.2).
 int make_grid(const p3p_grid* g, GridDev* out) {
     if (!g) return fail(P3P_ERR_INVALID_ARGUMENT, "grid is null");

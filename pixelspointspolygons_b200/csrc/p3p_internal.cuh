@@ -202,6 +202,7 @@ int launch_nchw_to_nhwc16(const float* x, int B, int C, int H, int W, int precis
 int launch_upsample_bilinear_nhwc16(const float* x, int B, int h, int w, int C, int64_t src_batch_stride, int H, int W, int precision,
                                     void* out, cudaStream_t st);
 int device_sm_count();
+size_t device_smem_optin();  // shared memory one CTA may opt in to, static + dynamic (cudaDevAttrMaxSharedMemoryPerBlockOptin)
 
 // ----------------------------------------------------------------------------------------------
 // device helpers

@@ -41,6 +41,7 @@ namespace p3p {
 namespace {
 
 constexpr int kTrainMaxM = 512;
+constexpr int kTrainMaxC = 512;  // thread = channel kernels: one CTA of at most 512 threads; back2 covers c and c + 256
 constexpr int kXS = 36;  // floats per x0 / yh0 row in shared memory (16-byte aligned rows: broadcast float4 loads)
 
 struct TrainLayout {
@@ -192,6 +193,29 @@ __device__ __forceinline__ Smem carve(float* base, int M, bool want_yh) {
 }
 size_t smem_floats(int M, bool want_yh) { return (size_t)M * 8 + (size_t)(M + 1) * kXS * (want_yh ? 2 : 1) + 256 + 6 * 32 + 32 + 96 + 3 * 512; }
 
+constexpr int kStats0Acc = 45;  // static float64 accumulators of train_stats0_kernel: rows, s[8], upper triangle of S
+
+// Dynamic shared memory (bytes) of every per-pillar kernel of the step, in one place: the launches take their sizes from
+// here, and fill_args refuses a (C, M) that any of them could not launch before an entry point does anything.
+struct TrainSmem {
+    size_t stats0, centre, stats1, forward, back1, back2;
+    size_t max_block;  // the largest dynamic + static shared memory of one CTA among them
+};
+TrainSmem train_smem(int M, int C) {
+    TrainSmem t;
+    const size_t base = smem_floats(M, false) * 4;
+    t.stats0 = base;
+    t.centre = base;
+    t.stats1 = base + 64 * sizeof(float);                  // + the centre of the layer-1 moments
+    t.forward = base;
+    t.back1 = base + (size_t)64 * C * sizeof(float);       // + A1s, the sparse dW1 block of the CTA
+    const size_t fl = smem_floats(M, false) + (size_t)(M + 1) * 33 + 3 * (size_t)C + 32 + 64 + 64 + 32 * 64;
+    t.back2 = (fl + 8 * 32 * 10 + (size_t)M + 2 + C) * 4;  // see the carve-up at the top of train_back2_kernel
+    t.max_block = t.stats0 + kStats0Acc * sizeof(double);
+    for (size_t v : {t.centre, t.stats1, t.forward, t.back1, t.back2}) t.max_block = v > t.max_block ? v : t.max_block;
+    return t;
+}
+
 // layer-0 constants of the batch into shared memory (bn0 must be final)
 __device__ __forceinline__ void load_layer0(const TrainArgs& a, const Smem& s) {
     const double* bn0 = a.st + a.tl.bn0;
@@ -313,9 +337,9 @@ __device__ __forceinline__ double warp_sum_d(double v) {
 __global__ void __launch_bounds__(256) train_stats0_kernel(TrainArgs a) {
     extern __shared__ __align__(16) float smem_f[];
     const Smem s = carve(smem_f, a.g.M, false);
-    __shared__ double acc[45];
+    __shared__ double acc[kStats0Acc];
     const int tid = threadIdx.x;
-    if (tid < 45) acc[tid] = 0.0;
+    if (tid < kStats0Acc) acc[tid] = 0.0;
     float m1[8], m2[36];
 #pragma unroll
     for (int i = 0; i < 8; ++i) m1[i] = 0.f;
@@ -880,15 +904,25 @@ __global__ void train_grads_kernel(const float* __restrict__ W, const float* __r
     }
 }
 
+int check_channels(int C) {
+    if (C < 1 || C > kTrainMaxC) return fail(P3P_ERR_UNSUPPORTED, "training kernels cover 1..%d channels, got %d", kTrainMaxC, C);
+    return P3P_OK;
+}
+
 int fill_args(TrainArgs* a, const p3p_grid* grid, int B, int64_t total, const p3p_pfn_params* p, double* state, void* ws, size_t ws_bytes) {
     if (!grid || !p || !state) return fail(P3P_ERR_INVALID_ARGUMENT, "null grid, params or state");
     if (!p->linear0_weight || !p->norm0_weight || !p->norm0_bias || !p->linear1_weight || !p->norm1_weight || !p->norm1_bias)
         return fail(P3P_ERR_INVALID_ARGUMENT, "null weight pointer");
-    if (p->channels < 1 || p->channels > 512) return fail(P3P_ERR_UNSUPPORTED, "training kernels cover 1..512 channels, got %d", p->channels);
+    int rc = check_channels(p->channels);
+    if (rc) return rc;
     memset(a, 0, sizeof(*a));
-    int rc = make_grid(grid, &a->g);
+    rc = make_grid(grid, &a->g);
     if (rc) return rc;
     if (a->g.M > kTrainMaxM) return fail(P3P_ERR_UNSUPPORTED, "training kernels cover max_points <= %d, got %d", kTrainMaxM, a->g.M);
+    const size_t need = train_smem(a->g.M, p->channels).max_block, cap = device_smem_optin();
+    if (need > cap)
+        return fail(P3P_ERR_UNSUPPORTED, "training kernels need %zu bytes of shared memory per CTA at max_points %d, channels %d; "
+                    "the device allows %zu", need, a->g.M, p->channels, cap);
     if (B < 0 || (int64_t)B * a->g.Vmax > 0x7fffffff) return fail(P3P_ERR_INVALID_ARGUMENT, "num_tiles %d", B);
     if (ws) {
         WsLayout l;
@@ -908,9 +942,9 @@ int fill_args(TrainArgs* a, const p3p_grid* grid, int B, int64_t total, const p3
     return P3P_OK;
 }
 
+// (fill_args has checked every size against the device's opt-in limit)
 template <typename K>
 int opt_in(K kernel, size_t smem) {
-    if (smem > 220 * 1024) return fail(P3P_ERR_UNSUPPORTED, "training kernel needs %zu bytes of shared memory", smem);
     P3P_CUDA_CHECK(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     return P3P_OK;
 }
@@ -929,7 +963,7 @@ using namespace p3p;
 extern "C" {
 
 int64_t p3p_pfn_train_state_doubles(int32_t channels, int64_t* offsets) {
-    if (channels < 1 || channels > 512) return 0;
+    if (check_channels(channels)) return 0;
     const TrainLayout l = make_train_layout(channels);
     if (offsets) {
         const int64_t o[14] = {l.mom0, l.sums0, l.bn0, l.mom1, l.sums1, l.bn1, l.cen, l.back1, l.back1g, l.A1, l.kq, l.back0, l.back0g, l.A0};
@@ -952,7 +986,7 @@ int p3p_pfn_train_stats0(const p3p_grid* grid, int32_t num_tiles, int64_t total_
     if (!workspace) return fail(P3P_ERR_INVALID_ARGUMENT, "workspace is null");
     cudaStream_t st = static_cast<cudaStream_t>(stream);
     P3P_CUDA_CHECK(cudaMemsetAsync(state, 0, (size_t)a.tl.total * sizeof(double), st));
-    const size_t smem = smem_floats(a.g.M, false) * 4;
+    const size_t smem = train_smem(a.g.M, a.C).stats0;
     rc = opt_in(train_stats0_kernel, smem);
     if (rc) return rc;
     if (num_tiles > 0) {
@@ -973,14 +1007,14 @@ int p3p_pfn_train_stats1(const p3p_grid* grid, int32_t num_tiles, int64_t total_
     if (!workspace) return fail(P3P_ERR_INVALID_ARGUMENT, "workspace is null");
     cudaStream_t st = static_cast<cudaStream_t>(stream);
     train_bn_kernel<<<1, 32, 0, st>>>(state + a.tl.sums0, 32, state + a.tl.bn0, nullptr, nullptr);
-    const size_t smem = smem_floats(a.g.M, false) * 4;
-    rc = opt_in(train_stats1_kernel, smem + 64 * sizeof(float));
+    const TrainSmem sm = train_smem(a.g.M, a.C);
+    rc = opt_in(train_stats1_kernel, sm.stats1);
     if (rc) return rc;
-    rc = opt_in(train_centre_kernel, smem);
+    rc = opt_in(train_centre_kernel, sm.centre);
     if (rc) return rc;
     if (num_tiles > 0) {
-        train_centre_kernel<<<kCentreCtas, 256, smem, st>>>(a);
-        train_stats1_kernel<<<grid_size(num_tiles, a.g.Vmax, 3), 256, smem + 64 * sizeof(float), st>>>(a);
+        train_centre_kernel<<<kCentreCtas, 256, sm.centre, st>>>(a);
+        train_stats1_kernel<<<grid_size(num_tiles, a.g.Vmax, 3), 256, sm.stats1, st>>>(a);
         train_uncentre_kernel<<<1, 1024, 0, st>>>(a);
     }
     const double* mom = state + a.tl.mom1;
@@ -992,7 +1026,8 @@ int p3p_pfn_train_stats1(const p3p_grid* grid, int32_t num_tiles, int64_t total_
 int p3p_pfn_train_stats2(const p3p_pfn_params* params, double* state, float* mean0, float* var0, float* mean1, float* var1,
                          void* stream) {
     if (!params || !state || !mean0 || !var0 || !mean1 || !var1) return fail(P3P_ERR_INVALID_ARGUMENT, "null pointer");
-    if (params->channels < 1 || params->channels > 512) return fail(P3P_ERR_UNSUPPORTED, "channels %d", params->channels);
+    const int rc = check_channels(params->channels);
+    if (rc) return rc;
     const TrainLayout l = make_train_layout(params->channels);
     cudaStream_t st = static_cast<cudaStream_t>(stream);
     train_bn_kernel<<<1, 32, 0, st>>>(state + l.sums0, 32, state + l.bn0, mean0, var0);
@@ -1019,7 +1054,7 @@ int p3p_pfn_train_forward(const p3p_grid* grid, int32_t num_tiles, int64_t total
     train_bn_kernel<<<(a.C + 127) / 128, 128, 0, st>>>(state + a.tl.sums1, a.C, state + a.tl.bn1, nullptr, nullptr);
     P3P_CUDA_CHECK(cudaMemsetAsync(out, 0, (size_t)num_tiles * a.g.ny * a.g.nx * a.C * sizeof(float), st));  // empty cells
     const int threads = a.C <= 256 ? 256 : (a.C + 31) / 32 * 32;
-    const size_t smem = smem_floats(a.g.M, false) * 4;
+    const size_t smem = train_smem(a.g.M, a.C).forward;
     rc = opt_in(train_forward_kernel, smem);
     if (rc) return rc;
     if (num_tiles > 0) train_forward_kernel<<<grid_size(num_tiles, a.g.Vmax, 1), threads, smem, st>>>(a);
@@ -1040,7 +1075,7 @@ int p3p_pfn_backward1(const p3p_grid* grid, int32_t num_tiles, int64_t total_poi
     const size_t zero_from = (size_t)a.tl.back1, zero_to = (size_t)a.tl.total;  // every backward accumulator
     P3P_CUDA_CHECK(cudaMemsetAsync(state + zero_from, 0, (zero_to - zero_from) * sizeof(double), st));
     const int threads = a.C <= 256 ? 256 : (a.C + 31) / 32 * 32;
-    const size_t smem = (smem_floats(a.g.M, false) + (size_t)64 * a.C) * 4;
+    const size_t smem = train_smem(a.g.M, a.C).back1;
     rc = opt_in(train_back1_kernel, smem);
     if (rc) return rc;
     if (num_tiles > 0) train_back1_kernel<<<grid_size(num_tiles, a.g.Vmax, 1), threads, smem, st>>>(a);
@@ -1058,8 +1093,7 @@ int p3p_pfn_backward2(const p3p_grid* grid, int32_t num_tiles, int64_t total_poi
     set_route(&a, const_cast<void*>(route), num_tiles);
     train_kq_kernel<<<65, 64, (size_t)a.C * sizeof(double), st>>>(a);
     train_kq2_kernel<<<1, 64, 0, st>>>(a);
-    const size_t fl = smem_floats(a.g.M, false) + (size_t)(a.g.M + 1) * 33 + 3 * (size_t)a.C + 32 + 64 + 64 + 32 * 64;
-    const size_t smem = (fl + 8 * 32 * 10 + a.g.M + 2 + a.C) * 4;
+    const size_t smem = train_smem(a.g.M, a.C).back2;
     rc = opt_in(train_back2_kernel, smem);
     if (rc) return rc;
     if (num_tiles > 0) train_back2_kernel<<<grid_size(num_tiles, a.g.Vmax, 2), 256, smem, st>>>(a);
@@ -1071,7 +1105,8 @@ int p3p_pfn_backward3(const p3p_pfn_params* params, const double* state, float* 
                       float* d_norm0_bias, float* d_linear1, float* d_norm1_weight, float* d_norm1_bias, void* stream) {
     if (!params || !state || !d_linear0 || !d_norm0_weight || !d_norm0_bias || !d_linear1 || !d_norm1_weight || !d_norm1_bias)
         return fail(P3P_ERR_INVALID_ARGUMENT, "null pointer");
-    if (params->channels < 1 || params->channels > 512) return fail(P3P_ERR_UNSUPPORTED, "channels %d", params->channels);
+    const int rc = check_channels(params->channels);
+    if (rc) return rc;
     const TrainLayout l = make_train_layout(params->channels);
     cudaStream_t st = static_cast<cudaStream_t>(stream);
     const double* m0 = state + l.mom0;

@@ -50,12 +50,15 @@ def exchange(t: torch.Tensor, group) -> None:
 
 
 def update_running_stats(norm: nn.Module, mean: torch.Tensor, var_biased: torch.Tensor, rows: torch.Tensor) -> None:
-    """What nn.BatchNorm1d.forward does to its buffers in train mode (momentum update with the unbiased variance)."""
+    """What nn.BatchNorm1d.forward does to its buffers in train mode (momentum update with the unbiased variance).  A batch
+    without a single row (no pillar on any rank) counts in num_batches_tracked but leaves the running statistics as they
+    are, as torch's batch_norm does for an empty input; `rows` stays on the device, so this costs no synchronisation."""
     if not getattr(norm, "track_running_stats", True) or norm.running_mean is None:
         return
     with torch.no_grad():
         norm.num_batches_tracked += 1
         m = norm.momentum if norm.momentum is not None else 1.0 / norm.num_batches_tracked.to(torch.float64)
+        m = (rows > 0).to(torch.float64) * m
         unbiased = var_biased.to(torch.float64) * (rows / torch.clamp(rows - 1.0, min=1.0))
         norm.running_mean.mul_(1.0 - m).add_((mean.to(torch.float64) * m).to(norm.running_mean.dtype))
         norm.running_var.mul_(1.0 - m).add_((unbiased * m).to(norm.running_var.dtype))

@@ -140,6 +140,26 @@ def test_update_running_stats_is_batchnorm1d_train_mode():
     assert p3p_train.sync_group(bn) is None and p3p_train.sync_group(nn.SyncBatchNorm(6)) is None  # no process group here
 
 
+@pytest.mark.parametrize("momentum", [0.01, None])
+def test_update_running_stats_on_an_empty_batch_is_batchnorm1d_train_mode(momentum):
+    """No row in the batch: torch's BatchNorm1d counts the batch but keeps its running statistics (and writes no NaN)."""
+    g = torch.Generator().manual_seed(1)
+    ref = nn.BatchNorm1d(6, eps=1e-3, momentum=momentum).train()
+    bn = nn.BatchNorm1d(6, eps=1e-3, momentum=momentum).train()
+    for m in (ref, bn):
+        m.running_mean.copy_(torch.randn(6, generator=g))
+        m.running_var.copy_(torch.rand(6, generator=g) + 0.5)
+    bn.load_state_dict(ref.state_dict())
+    ref(torch.zeros(0, 6))
+    p3p_train.update_running_stats(bn, torch.zeros(6), torch.zeros(6), torch.tensor(0.0, dtype=torch.float64))
+    assert torch.equal(bn.running_mean, ref.running_mean) and torch.equal(bn.running_var, ref.running_var)
+    assert int(bn.num_batches_tracked) == int(ref.num_batches_tracked) == 1
+    x = torch.randn(30, 6, generator=g)  # and the next, non-empty batch is counted as the second
+    ref(x)
+    p3p_train.update_running_stats(bn, x.mean(0), x.var(0, unbiased=False), torch.tensor(30.0, dtype=torch.float64))
+    assert torch.allclose(bn.running_mean, ref.running_mean, atol=1e-7) and torch.allclose(bn.running_var, ref.running_var, atol=1e-7)
+
+
 def _free_port():
     with socket.socket() as s:
         s.bind(("127.0.0.1", 0))
