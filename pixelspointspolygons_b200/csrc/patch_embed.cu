@@ -195,6 +195,11 @@ __global__ void __launch_bounds__(kPeThreads, 1) patch_embed_tc_kernel(PeArgs a)
         }
     };
     const int quad = warp & 3, hi_half = warp >> 2;
+    // The fp32 NCHW epilogue stages its transposes in a weight tile's space, 8 warps x 32 x 17 floats.  A 16-bit tile of one
+    // input channel is 16 KB, smaller than that: past its end lie the next tile, still under its MMAs, or the image operand,
+    // which a further round reads again.  Such tiles store their 16 cells per thread directly.
+    const bool stage_nchw = a.out_layout == P3P_LAYOUT_NCHW && a.out_dtype == P3P_DTYPE_F32 &&
+                            a_tile_bytes >= (size_t)kPeThreads * 17 * sizeof(float);
     const int nblk = a.N / 16, split = (nblk + 1) / 2;
     const int blk0 = hi_half ? split : 0, blk1 = hi_half ? nblk : split;
     uint32_t tmem_base = 0;
@@ -254,7 +259,7 @@ __global__ void __launch_bounds__(kPeThreads, 1) patch_embed_tc_kernel(PeArgs a)
             for (int blk = blk0; blk < blk1; ++blk) {
                 float v[16];
                 tmem_ld16_wait(tmem_base + ((uint32_t)(quad * 32) << 16) + (uint32_t)(t * 128 + blk * 16), v);
-                if (a.out_layout == P3P_LAYOUT_NCHW && a.out_dtype == P3P_DTYPE_F32) {
+                if (stage_nchw) {
                     // The thread holds 16 consecutive cells (64 bytes) of ITS channel: stored as they are, one instruction
                     // touches 32 cache lines.  Through a per-warp transpose in shared memory (the weight tile's space: its
                     // MMAs are done) a quarter-warp writes the 64 bytes of one channel, 8 channels = 8 lines per instruction.
@@ -280,7 +285,11 @@ __global__ void __launch_bounds__(kPeThreads, 1) patch_embed_tc_kernel(PeArgs a)
                         const int64_t r0 = ((int64_t)b * a.ny * a.nx + (int64_t)cy0 * a.nx + blk * 16) * a.c_total + a.c_offset + ch;
 #pragma unroll
                         for (int i = 0; i < 16; ++i) store_out(a.out, a.out_dtype, r0 + (int64_t)i * a.c_total, v[i] + bv);
-                        } else {
+                    } else if (a.out_dtype == P3P_DTYPE_F32) {
+                        float* dst = static_cast<float*>(a.out) + row0 + blk * 16;
+#pragma unroll
+                        for (int i = 0; i < 16; ++i) dst[i] = v[i] + bv;
+                    } else {
                         unsigned short* dst = static_cast<unsigned short*>(a.out) + row0 + blk * 16;
 #pragma unroll
                         for (int i = 0; i < 16; ++i) dst[i] = to_16bit(v[i] + bv, a.out_dtype);
