@@ -60,9 +60,6 @@ struct ConvArgs {
     const float* pos_embed;  // ((1 + H W), Cout)       ViT-token epilogue only
 };
 
-__device__ __forceinline__ void mbar_expect_tx(uint64_t* bar, uint32_t bytes) {
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes) : "memory");
-}
 __device__ __forceinline__ void tma_load_4d(uint32_t dst, const CUtensorMap* tm, uint64_t* bar, int c0, int c1, int c2, int c3) {
     asm volatile(
         "cp.async.bulk.tensor.4d.shared::cluster.global.tile.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5, %6}], [%2];"
@@ -73,15 +70,6 @@ __device__ __forceinline__ void tma_load_2d(uint32_t dst, const CUtensorMap* tm,
     asm volatile(
         "cp.async.bulk.tensor.2d.shared::cluster.global.tile.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4}], [%2];"
         ::"r"(dst), "l"(tm), "r"(smem_u32(bar)), "r"(c0), "r"(c1)
-        : "memory");
-}
-__device__ __forceinline__ void tmem_ld16(uint32_t taddr, float (&v)[16]) {
-    asm volatile(
-        "tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15}, [%16];\n"
-        "tcgen05.wait::ld.sync.aligned;\n"
-        : "=f"(v[0]), "=f"(v[1]), "=f"(v[2]), "=f"(v[3]), "=f"(v[4]), "=f"(v[5]), "=f"(v[6]), "=f"(v[7]), "=f"(v[8]),
-          "=f"(v[9]), "=f"(v[10]), "=f"(v[11]), "=f"(v[12]), "=f"(v[13]), "=f"(v[14]), "=f"(v[15])
-        : "r"(taddr)
         : "memory");
 }
 
@@ -189,7 +177,7 @@ conv3x3_tc_kernel(const __grid_constant__ CUtensorMap tm_x, const __grid_constan
             const uint32_t taddr = tmem_base + ((uint32_t)(quad * 32) << 16) + (uint32_t)(t * a.acc_stride);
             for (int j0 = 0; j0 < a.N; j0 += 16) {
                 float v[16];
-                tmem_ld16(taddr + (uint32_t)j0, v);
+                tmem_ld16_wait(taddr + (uint32_t)j0, v);
 #pragma unroll
                 for (int i = 0; i < 16; ++i) {
                     v[i] += sh;

@@ -25,20 +25,12 @@ int fail(int code, const char* fmt, ...);
 // ----------------------------------------------------------------------------------------------
 constexpr int kFlagDropOverflow = P3P_GRID_DROP_OVERFLOW;  // DESIGN.md uncertainty ledger U1
 constexpr int kMaxKeys = 6144;        // smem histogram budget of the ranking kernels
-// voxelizer shape (build-time tunables): threads per CTA, CTAs per SM, points per lane; a chunk holds threads * points-per-lane
-// points and the whole batch should be ONE wave of CTAs (capi.cu sizes the chunks for that)
-#ifndef P3P_VOX_THREADS
-#define P3P_VOX_THREADS 256
-#endif
-#ifndef P3P_VOX_CTAS
-#define P3P_VOX_CTAS 3
-#endif
-#ifndef P3P_VOX_PPL
-#define P3P_VOX_PPL 16
-#endif
-constexpr int kVoxThreads = P3P_VOX_THREADS, kVoxCtasPerSm = P3P_VOX_CTAS;
+// voxelizer shape: a chunk holds threads * points-per-lane points and the whole batch should be ONE wave of CTAs (capi.cu
+// sizes the chunks for that).  The CTA shape does not matter (DESIGN 4.1: 512 x 2 x 12 and 384 x 2 x 16 measured no faster).
+constexpr int kVoxThreads = 256;                                // threads per CTA
+constexpr int kVoxCtasPerSm = 3;                                // CTAs per SM
 constexpr int kChunkGranule = 4 * kVoxThreads;                  // every lane owns whole groups of 4 points
-constexpr int kMaxChunkPoints = kVoxThreads * P3P_VOX_PPL;      // points per ranking chunk held in registers
+constexpr int kMaxChunkPoints = kVoxThreads * 16;               // points per ranking chunk held in registers (16 per lane)
 constexpr int kC0 = 32;               // feat_channels[0] / 2: width of PFN layer 0
 
 struct GridDev {
@@ -288,19 +280,6 @@ __device__ __forceinline__ void mbar_init(uint64_t* bar, uint32_t count) {
 __device__ __forceinline__ void mbar_arrive(uint64_t* bar) {
     asm volatile("{.reg .b64 st; mbarrier.arrive.shared::cta.b64 st, [%0];}" ::"r"(smem_u32(bar)) : "memory");
 }
-__device__ __forceinline__ bool mbar_try_wait(uint64_t* bar, uint32_t parity) {
-    uint32_t ok;
-    asm volatile(
-        "{.reg .pred p; mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2; selp.u32 %0, 1, 0, p;}"
-        : "=r"(ok)
-        : "r"(smem_u32(bar)), "r"(parity)
-        : "memory");
-    return ok != 0;
-}
-__device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity) {
-    while (!mbar_try_wait(bar, parity)) {
-    }
-}
 // plain shared-memory accesses by 32-bit shared address (no generic-pointer arithmetic in the hot loops)
 __device__ __forceinline__ float lds_f32(uint32_t addr) {
     float v;
@@ -334,6 +313,12 @@ __device__ __forceinline__ bool mbar_try_wait_sa(uint32_t bar, uint32_t parity) 
 __device__ __forceinline__ void mbar_wait_sa(uint32_t bar, uint32_t parity) {
     while (!mbar_try_wait_sa(bar, parity)) {
     }
+}
+__device__ __forceinline__ bool mbar_try_wait(uint64_t* bar, uint32_t parity) { return mbar_try_wait_sa(smem_u32(bar), parity); }
+__device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity) { mbar_wait_sa(smem_u32(bar), parity); }
+// arrive and expect `bytes` of async-copy transactions (TMA / bulk copies completing on the barrier)
+__device__ __forceinline__ void mbar_expect_tx(uint64_t* bar, uint32_t bytes) {
+    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes) : "memory");
 }
 __device__ __forceinline__ uint32_t mbar_test_sa(uint32_t bar, uint32_t parity) {
     uint32_t ok;
@@ -395,36 +380,20 @@ __device__ __forceinline__ uint32_t make_idesc(int fmt_code, int m, int n) {
     return (1u << 4) | (fmt << 7) | (fmt << 10) | ((uint32_t)(n >> 3) << 17) | ((uint32_t)(m >> 4) << 24);
 }
 // tcgen05.ld + tcgen05.wait::ld in ONE asm statement: the destination registers are only defined once the wait has
-// retired, so no consumer can be scheduled between the load and the wait.  (ptxas tracks the load's registers with a
-// scoreboard, so loads into distinct registers still overlap with the arithmetic on earlier ones.)
-__device__ __forceinline__ void tmem_ld32_wait(uint32_t taddr, float (&v)[32]) {
+// retired, so no consumer can be scheduled between the load and the wait.
+__device__ __forceinline__ void tmem_ld16_wait(uint32_t taddr, float (&v)[16]) {
     asm volatile(
-        "tcgen05.ld.sync.aligned.32x32b.x32.b32 {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15,%16,%17,%18,%19,%20,%21,%22,%23,%24,%25,%26,%27,%28,%29,%30,%31}, [%32];\n"
+        "tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15}, [%16];\n"
         "tcgen05.wait::ld.sync.aligned;\n"
-        : "=f"(v[0]),"=f"(v[1]),"=f"(v[2]),"=f"(v[3]),"=f"(v[4]),"=f"(v[5]),"=f"(v[6]),"=f"(v[7]),"=f"(v[8]),"=f"(v[9]),"=f"(v[10]),"=f"(v[11]),"=f"(v[12]),"=f"(v[13]),"=f"(v[14]),"=f"(v[15]),"=f"(v[16]),"=f"(v[17]),"=f"(v[18]),"=f"(v[19]),"=f"(v[20]),"=f"(v[21]),"=f"(v[22]),"=f"(v[23]),"=f"(v[24]),"=f"(v[25]),"=f"(v[26]),"=f"(v[27]),"=f"(v[28]),"=f"(v[29]),"=f"(v[30]),"=f"(v[31])
+        : "=f"(v[0]), "=f"(v[1]), "=f"(v[2]), "=f"(v[3]), "=f"(v[4]), "=f"(v[5]), "=f"(v[6]), "=f"(v[7]), "=f"(v[8]),
+          "=f"(v[9]), "=f"(v[10]), "=f"(v[11]), "=f"(v[12]), "=f"(v[13]), "=f"(v[14]), "=f"(v[15])
         : "r"(taddr)
         : "memory");
 }
-
 // Split form for software pipelining inside a warp: issue a load, then later wait for every outstanding load of the
 // thread.  The wait lists the registers of the load(s) it completes as in/out operands so that no consumer can be
 // scheduled above it; ptxas tracks tcgen05.ld with a scoreboard, so arithmetic on registers of an EARLIER, already
 // awaited load overlaps with a load that is still in flight.
-#define P3P_R32(v)                                                                                                        \
-    "+f"(v[0]),"+f"(v[1]),"+f"(v[2]),"+f"(v[3]),"+f"(v[4]),"+f"(v[5]),"+f"(v[6]),"+f"(v[7]),"+f"(v[8]),"+f"(v[9]),"+f"(v[10]),   \
-    "+f"(v[11]),"+f"(v[12]),"+f"(v[13]),"+f"(v[14]),"+f"(v[15]),"+f"(v[16]),"+f"(v[17]),"+f"(v[18]),"+f"(v[19]),"+f"(v[20]),    \
-    "+f"(v[21]),"+f"(v[22]),"+f"(v[23]),"+f"(v[24]),"+f"(v[25]),"+f"(v[26]),"+f"(v[27]),"+f"(v[28]),"+f"(v[29]),"+f"(v[30]),    \
-    "+f"(v[31])
-__device__ __forceinline__ void tmem_ld32_issue(uint32_t taddr, float (&v)[32]) {
-    asm volatile(
-        "tcgen05.ld.sync.aligned.32x32b.x32.b32 {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15,%16,%17,%18,%19,%20,%21,%22,%23,%24,%25,%26,%27,%28,%29,%30,%31}, [%32];\n"
-        : "=f"(v[0]),"=f"(v[1]),"=f"(v[2]),"=f"(v[3]),"=f"(v[4]),"=f"(v[5]),"=f"(v[6]),"=f"(v[7]),"=f"(v[8]),"=f"(v[9]),"=f"(v[10]),"=f"(v[11]),"=f"(v[12]),"=f"(v[13]),"=f"(v[14]),"=f"(v[15]),"=f"(v[16]),"=f"(v[17]),"=f"(v[18]),"=f"(v[19]),"=f"(v[20]),"=f"(v[21]),"=f"(v[22]),"=f"(v[23]),"=f"(v[24]),"=f"(v[25]),"=f"(v[26]),"=f"(v[27]),"=f"(v[28]),"=f"(v[29]),"=f"(v[30]),"=f"(v[31])
-        : "r"(taddr)
-        : "memory");
-}
-__device__ __forceinline__ void tmem_ld_wait(float (&v)[32]) {
-    asm volatile("tcgen05.wait::ld.sync.aligned;\n" : P3P_R32(v) : : "memory");
-}
 #define P3P_R16(v)                                                                                                        \
     "+f"(v[0]),"+f"(v[1]),"+f"(v[2]),"+f"(v[3]),"+f"(v[4]),"+f"(v[5]),"+f"(v[6]),"+f"(v[7]),"+f"(v[8]),"+f"(v[9]),"+f"(v[10]),   \
     "+f"(v[11]),"+f"(v[12]),"+f"(v[13]),"+f"(v[14]),"+f"(v[15])
@@ -437,16 +406,6 @@ __device__ __forceinline__ void tmem_ld16_issue(uint32_t taddr, float (&v)[16]) 
 }
 __device__ __forceinline__ void tmem_ld_wait16(float (&v)[16]) {
     asm volatile("tcgen05.wait::ld.sync.aligned;\n" : P3P_R16(v) : : "memory");
-}
-// non-blocking probe of an mbarrier phase (the result is consumed later: its latency hides behind independent work)
-__device__ __forceinline__ uint32_t mbar_test(uint64_t* bar, uint32_t parity) {
-    uint32_t ok;
-    asm volatile(
-        "{.reg .pred p; mbarrier.test_wait.parity.shared::cta.b64 p, [%1], %2; selp.u32 %0, 1, 0, p;}"
-        : "=r"(ok)
-        : "r"(smem_u32(bar)), "r"(parity)
-        : "memory");
-    return ok;
 }
 
 __device__ __forceinline__ float fmax3(float a, float b, float c) {

@@ -101,16 +101,6 @@ __device__ __forceinline__ void put_run(unsigned char* tile, int nrows, int row,
     }
 }
 
-__device__ __forceinline__ void tmem_ld16_wait(uint32_t taddr, float (&v)[16]) {
-    asm volatile(
-        "tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15}, [%16];\n"
-        "tcgen05.wait::ld.sync.aligned;\n"
-        : "=f"(v[0]), "=f"(v[1]), "=f"(v[2]), "=f"(v[3]), "=f"(v[4]), "=f"(v[5]), "=f"(v[6]), "=f"(v[7]), "=f"(v[8]),
-          "=f"(v[9]), "=f"(v[10]), "=f"(v[11]), "=f"(v[12]), "=f"(v[13]), "=f"(v[14]), "=f"(v[15])
-        : "r"(taddr)
-        : "memory");
-}
-
 // CTA = (row group of R cell rows, image): the B operand (the pixel runs of the row group, the only HBM read) is built ONCE
 // and multiplied with every 128-channel tile of the weights -- kTilesResident tiles at a time (all three of C = 384 with
 // 16-bit operands; one with tf32, whose tiles are twice as large), each tile an MMA chain into its own TMEM columns with its
@@ -214,7 +204,7 @@ __global__ void __launch_bounds__(kPeThreads, 1) patch_embed_tc_kernel(PeArgs a)
             // the tiles are stored as their shared-memory operand images: one bulk copy per tile (TMA, no register
             // traffic) next to the threads' work on the pixel runs
             if (tid == 0) {
-                asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(&abar)), "r"((uint32_t)(ntiles * a_tile_bytes)) : "memory");
+                mbar_expect_tx(&abar, (uint32_t)(ntiles * a_tile_bytes));
                 for (int t = 0; t < ntiles; ++t)
                     asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(smem_u32(sA + (size_t)t * a_tile_bytes)),
                                  "l"(a.blob + (size_t)(mt0 + t) * a_tile_bytes), "r"((uint32_t)a_tile_bytes), "r"(smem_u32(&abar)) : "memory");

@@ -358,50 +358,11 @@ constexpr int kMmaWarps = 4;                   // warp group 0: warp m < 3 issue
 constexpr int kEpiWarp0 = kMmaWarps + kNF;     // then kNF front-end warps, then the epilogue warps
 constexpr int kEpiGroups = 3;                  // epilogue groups of 4 warps (one warp per TMEM lane quarter)
 constexpr int kTcThreads = 32 * (kEpiWarp0 + 4 * kEpiGroups);
-// P3P_EPI4 (build-time switch, compile-time modes 1-3 only): FOUR epilogue groups.  One warp reads TMEM at 45 B/clk whatever
-// the load width, so the only way to drain faster is more warps draining at once.  Pillar q of a unit's 8 goes to group
-// (m + q) mod 4 for channel tile m: a pillar's three tiles land on three different groups, every group does 3 jobs per 4
-// pillars.  28 warps x 72 registers at launch; the epilogue warps drop to 64 (two x16 buffers still fit without spills).
-// Measured (B = 16, fp16, parity-green on the whole suite): PFN 42.0 -> 52.1 us (56 registers: 55.3 us), step 53.7 -> 63.4 us:
-// sixteen draining warps take the issue slots the front end needs (7 warps per scheduler).  Off; kept for the record.
-#ifndef P3P_EPI4
-#define P3P_EPI4 0
-#endif
-constexpr int kEpiGroupsMax = 4;
-template <int kMode> constexpr bool kFourGroups = (P3P_EPI4 != 0) && (kMode != 0);
-template <int kMode> constexpr int kThreadsOf = 32 * (kEpiWarp0 + 4 * (kFourGroups<kMode> ? 4 : kEpiGroups));
-#ifndef P3P_REG_EPI4
-#define P3P_REG_EPI4 64
-#endif
-constexpr int kRegEpi4 = P3P_REG_EPI4;
 
-#ifndef P3P_NS_16
-#define P3P_NS_16 8
-#define P3P_NS_TF32 4
-#endif
-#ifndef P3P_REG_MMA
-#define P3P_REG_MMA 40
-#define P3P_REG_FRONT 104
-#define P3P_REG_EPI 72
-#endif
-constexpr int kRegMma = P3P_REG_MMA, kRegFront = P3P_REG_FRONT, kRegEpi = P3P_REG_EPI;  // registers per thread after setmaxnreg (launch: 80)
+constexpr int kRegMma = 40, kRegFront = 104, kRegEpi = 72;  // registers per thread after setmaxnreg (launch: 80)
 // setmaxnreg redistributes the CTA's OWN launch allocation (24 warps x 80 registers), not the SM's spare registers: a split
 // that exceeds it leaves the last warps spinning in the allocation forever
 static_assert(4 * kRegMma + 8 * kRegFront + 12 * kRegEpi <= 24 * 80, "register pool of the launch exceeded");
-static_assert(!P3P_EPI4 || 4 * kRegMma + 8 * kRegFront + 16 * kRegEpi4 <= 28 * 72, "register pool of the four-group launch exceeded");
-// Two epilogue schedules that were measured and did NOT pay (B = 16, fp16, kernel time): issuing the next pillar's first
-// load before the last maximum of the current one (P3P_EPI_PIPE: 41.9 -> 43.4 us) and running a unit's tail behind the
-// next unit's first pair (P3P_EPI_DEFER: -> 46.7 us; the accumulator stages are refilled during the tail either way).
-// Kept behind switches for the record; the double-buffered W1b'hmax accumulators / maxima strips they need stay.
-#ifndef P3P_EPI_PIPE
-#define P3P_EPI_PIPE 0
-#endif
-#ifndef P3P_EPI_UNROLL
-#define P3P_EPI_UNROLL 1  // the unit's 4 pairs unrolled: barrier parities and strip offsets become constants of the body (r02: PFN 42.2 -> 41.1 us)
-#endif
-#ifndef P3P_EPI_DEFER
-#define P3P_EPI_DEFER 0
-#endif
 constexpr int kUnit = 8;                       // items per unit = 4 pillar pairs, consecutive canvas cells
 constexpr int kPairsPerUnit = kUnit / 2;
 constexpr int kTiles = 3;                      // 128-channel MMA tiles (C <= 384)
@@ -423,10 +384,10 @@ struct TcCfg {
     static constexpr uint32_t kLayout = kTf32 ? 2u : 4u;  // SWIZZLE_128B : SWIZZLE_64B
     static constexpr uint32_t kSBO = 8 * RB;
     static constexpr int kKSteps = kTf32 ? 4 : 2;         // UMMA_K = 8 (tf32) / 16 (16-bit): 32 bytes per step
-    static constexpr int kNS = kTf32 ? P3P_NS_TF32 : P3P_NS_16;            // B-operand stages: pillar pairs in flight
+    static constexpr int kNS = kTf32 ? 4 : 8;             // B-operand stages: pillar pairs in flight
     static constexpr size_t kSmemOperands = (size_t)6 * kATile + (size_t)kNS * kHStage + 2 * (size_t)kGStage;
     static constexpr size_t kSmemFloats = 10 * 32 + 384 + kNF * 128 * 4;
-    static constexpr size_t kSmemBytes = kSmemOperands + kSmemFloats * 4 + (2 * kNS + 2 * kTiles * kAccStages + 4 * kTiles + 2 + 2 + 4 * kTiles) * 8 + 16 + 2 * kNF * 4 + 2 * kValidRing + 2 * 4 * kEpiGroupsMax * kUnit * 32 * 4 + 2 * kNF * 4 * 4 + 2 * kNF * 32 * 4;
+    static constexpr size_t kSmemBytes = kSmemOperands + kSmemFloats * 4 + (2 * kNS + 2 * kTiles * kAccStages + 4 * kTiles + 2 + 2) * 8 + 16 + 2 * kNF * 4 + 2 * kValidRing + 4 * kEpiGroups * kUnit * 32 * 4 + 2 * kNF * 4 * 4 + 2 * kNF * 32 * 4;
 };
 
 
@@ -513,10 +474,8 @@ __device__ __forceinline__ float max16_with(float prev, const float (&v)[16]) {
 // (B, 1 + ny nx, C) sequence with pos_embed added.  Modes 1-3 are the shipped encoder configurations with every run-time
 // branch of the steady-state loops resolved at compile time.
 template <int kPrec, int kMode>
-__global__ void __launch_bounds__(kThreadsOf<kMode>, 1) pfn_tc_kernel(PfnArgs a) {
+__global__ void __launch_bounds__(kTcThreads, 1) pfn_tc_kernel(PfnArgs a) {
     using Cfg = TcCfg<kPrec>;
-    constexpr int kTcThreads = kThreadsOf<kMode>;  // (shadows the three-group constant inside the kernel)
-    constexpr bool kFour = kFourGroups<kMode>;
     constexpr bool kTf32 = Cfg::kTf32;
     constexpr int kNS = Cfg::kNS;
     // The kernel has no static shared memory, so the dynamic block starts at shared-memory offset 0 of the CTA window and
@@ -538,12 +497,11 @@ __global__ void __launch_bounds__(kThreadsOf<kMode>, 1) pfn_tc_kernel(PfnArgs a)
     uint64_t* gt_full = t_empty + kTiles * kAccStages;  // [3 tiles][2 slots] MMA warp m -> epilogue group m, per unit (W1b' hmax accumulator)
     uint64_t* gt_empty = gt_full + 2 * kTiles;          // [3][2] epilogue group m -> MMA warp m (128 arrivals)
     uint64_t* g_empty = gt_empty + 2 * kTiles;          // [2] MMA warps -> front end: hmax rows of the unit slot consumed (MT commits)
-    uint64_t* t_full4 = g_empty + 2;                    // [3 tiles][4] four-group schedule: MMA warp m -> the group that drains pillar q, by q & 3
-    uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(t_full4 + 4 * kTiles);
+    uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(g_empty + 2);
     int* sDesc = reinterpret_cast<int*>(tmem_slot + 2);                 // [kNF][2] descriptor word of the item decoded next
     unsigned char* sValid = reinterpret_cast<unsigned char*>(sDesc + 2 * kNF);  // [kValidRing pairs][2]: the item holds a pillar
-    float* sRmax = reinterpret_cast<float*>(sValid + 2 * kValidRing);           // [12 epilogue warps][2 unit parities][kUnit][32]: pillar maxima
-    int* sBlkSum = reinterpret_cast<int*>(sRmax + 4 * kEpiGroupsMax * 2 * kUnit * 32);  // [2 unit parities][kNF][4] fixed-point sums of a block
+    float* sRmax = reinterpret_cast<float*>(sValid + 2 * kValidRing);           // [12 epilogue warps][kUnit][32]: pillar maxima of the unit in work
+    int* sBlkSum = reinterpret_cast<int*>(sRmax + 4 * kEpiGroups * kUnit * 32);  // [2 unit parities][kNF][4] fixed-point sums of a block
     uint32_t* sBlkMax = reinterpret_cast<uint32_t*>(sBlkSum + 2 * kNF * 4);          // [2][kNF][32] hmax of a block (32 words: fp32, or 16 packed)
 
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
@@ -563,9 +521,8 @@ __global__ void __launch_bounds__(kThreadsOf<kMode>, 1) pfn_tc_kernel(PfnArgs a)
     if (tid == 32) {
         for (int i = 0; i < kNS; ++i) { mbar_init(&h_full[i], 2); mbar_init(&h_empty[i], (uint32_t)MT); }
         for (int i = 0; i < kTiles * kAccStages; ++i) { mbar_init(&t_full[i], 1); mbar_init(&t_empty[i], 128); }
-        for (int i = 0; i < 2 * kTiles; ++i) { mbar_init(&gt_full[i], 1); mbar_init(&gt_empty[i], kFour ? 512 : 128); }  // (four groups: every group reads two columns of every tile's unit accumulator)
+        for (int i = 0; i < 2 * kTiles; ++i) { mbar_init(&gt_full[i], 1); mbar_init(&gt_empty[i], 128); }
         mbar_init(&g_empty[0], (uint32_t)MT); mbar_init(&g_empty[1], (uint32_t)MT);
-        for (int i = 0; i < 4 * kTiles; ++i) mbar_init(&t_full4[i], 1);
         fence_mbar_init();
     }
     {
@@ -635,10 +592,7 @@ __global__ void __launch_bounds__(kThreadsOf<kMode>, 1) pfn_tc_kernel(PfnArgs a)
                         for (int k = 0; k < Cfg::kKSteps; ++k)
                             tc_mma<kTf32>(d_tile + (uint32_t)(s * kAccCols), ((uint64_t)desc_hi << 32) | (a1_lo + (uint32_t)(k * 2)),
                                           ((uint64_t)desc_hi << 32) | (b_lo + (uint32_t)(k * 2)), idesc_main, k > 0);
-                        // four groups: pillar q = 2 p + s of tile m is drained by group (m + q) mod 4; a parity wait only tells
-                        // adjacent phases apart, so every group gets barriers of its own (indexed by q & 3) and sees each phase
-                        if constexpr (kFour) tc_commit(&t_full4[m * 4 + 2 * (p & 1) + s]);
-                        else tc_commit(&tf[s]);
+                        tc_commit(&tf[s]);
                     }
                     __syncwarp();
                 }
@@ -958,103 +912,9 @@ __global__ void __launch_bounds__(kThreadsOf<kMode>, 1) pfn_tc_kernel(PfnArgs a)
             PTL(1 + fw, j, 2);
             if (lane == 0) mbar_arrive(&h_full[st]);
         }
-    } else if (kFour) {
-        // =========================== epilogue, four groups (P3P_EPI4; modes 1-3) ===========================
-        // Pillar i of a unit, channel tile m -> group (m + i) mod 4, i.e. group g drains tile (g - i) mod 4 of pillar i and
-        // sits pillar i out when that is 3: three jobs per four pillars for every group, a pillar's three tiles on three
-        // different groups.  Barrier phases are those of the three-group schedule (they depend on the pillar, not on who
-        // drains it); the unit accumulators of every tile are read by all four groups (gt_empty counts 512).
-        if constexpr (kFour) {
-            setmaxnreg_dec<kRegEpi4>();
-            const int g = (warp - kEpiWarp0) >> 2;
-            const int quad = warp & 3;  // TMEM lanes this warp may read: 32 * (warp id % 4)
-            const bool f32 = (kMode == 2) || (kMode == 3) || (a.out_dtype == P3P_DTYPE_F32);
-            const int C = a.bl.C, ipt = a.items_per_tile;
-            const uint32_t tlane = tmem_base + ((uint32_t)(quad * 32) << 16);
-            const int cl = quad * 32 + lane;  // channel inside a 128-channel tile
-            float b1v[3];
-#pragma unroll
-            for (int mm = 0; mm < 3; ++mm) b1v[mm] = sB1[mm * 128 + cl];
-            ItemWalk wu;  // position of the first item of the unit in work
-            wu.init(((int)blockIdx.x * kUnit) < total_items ? ((int)blockIdx.x * kUnit) : 0, (int)gridDim.x * kUnit, ipt);
-            const uint32_t tf_sa = opaque(smem_u32(t_full4)), te_sa = opaque(smem_u32(t_empty));
-            const uint32_t gtf_sa = opaque(smem_u32(gt_full)), gte_sa = opaque(smem_u32(gt_empty));
-            const uint32_t rmax_sa = opaque(smem_u32(sRmax + (warp - kEpiWarp0) * (2 * kUnit * 32) + lane));
-            const uint32_t valid_sa = opaque(smem_u32(sValid));
-            const int64_t rs = a.row_stride;
-            const int64_t rows_first = (int64_t)blockIdx.x * kUnit * rs + a.row_offset + cl;
-            float* rows_dst = static_cast<float*>(a.out) + rows_first;
-            unsigned short* rows_dst16 = static_cast<unsigned short*>(a.out) + rows_first;
-            const int64_t rows_step = (int64_t)gridDim.x * kUnit * rs;
-            float va[16], vb[16];
-            for (int j = 0; j < my_units; ++j) {
-                const int ub = wu.b, ur = wu.r;  // tile / position of the unit's first item
-                wu.step();
-#pragma unroll
-                for (int i = 0; i < kUnit; ++i) {
-                    const int m = (g - i) & 3;
-                    if (m < MT) {  // (MT <= 3: the group sits this pillar out when m == 3)
-                        // barrier (m, q & 3) completes once per four pillars: phase q >> 2 = 2 j + (i >> 2)
-                        const uint32_t bo = 8u * (uint32_t)(m * kAccStages + (i & 1));
-                        mbar_wait_sa(tf_sa + 8u * (uint32_t)(m * 4 + (i & 3)), (uint32_t)(i >> 2) & 1u);
-                        tc_fence_after();
-                        const uint32_t ta = tlane + (uint32_t)((m * kAccStages + (i & 1)) * kAccCols);
-                        tmem_ld16_issue(ta, va);
-                        tmem_ld_wait16(va);
-                        tmem_ld16_issue(ta + 16, vb);
-                        const float r0 = max16(va);
-                        tmem_ld_wait16(vb);
-                        tmem_ld16_issue(ta + 32, va);
-                        const float r1 = max16(vb);
-                        tmem_ld_wait16(va);
-                        tmem_ld16_issue(ta + 48, vb);
-                        const float r2 = max16(va);
-                        tmem_ld_wait16(vb);
-                        tc_fence_before();
-                        mbar_arrive_sa(te_sa + bo);
-                        sts_f32(rmax_sa + (uint32_t)(i * 128), fmaxf(fmax3(r0, r1, r2), max16(vb)));
-                    }
-                }
-                // ---- unit tail: + W1b' hmax + b1, relu, store; tile by tile (8 accumulator columns in registers at a time) ----
-                const uint2 vv = lds_u32x2(valid_sa + (uint32_t)(((j * kPairsPerUnit) & (kValidRing - 1)) * 2));
-#pragma unroll
-                for (int m = 0; m < kTiles; ++m) {
-                    if (m < MT) {
-                        float gv[8];
-                        const uint32_t bo = 8u * (uint32_t)(2 * m + (j & 1));
-                        mbar_wait_sa(gtf_sa + bo, ((uint32_t)j >> 1) & 1u);
-                        tc_fence_after();
-                        tmem_ld8_wait(tlane + (uint32_t)(kGCol0 + m * 16 + (j & 1) * kGSlotCols), gv);
-                        tc_fence_before();
-                        mbar_arrive_sa(gte_sa + bo);
-                        const int c = m * 128 + cl;
-#pragma unroll
-                        for (int i = 0; i < kUnit; ++i) {
-                            if (((g - i) & 3) == m && c < C) {
-                                const unsigned word = i < 4 ? vv.x : vv.y;
-                                const bool v = ((word >> (8 * (i & 3))) & 0xFFu) != 0;
-                                const float ob = v ? fmaxf(lds_f32(rmax_sa + (uint32_t)(i * 128)) + (gv[i] + b1v[m]), 0.f) : 0.f;
-                                if constexpr (kMode == 3) {
-                                    const int64_t row = (int64_t)ub * a.token_rows + 1 + ur + i;
-                                    static_cast<float*>(a.out)[row * C + c] = ob + __ldg(a.pos_embed + (int64_t)(1 + ur + i) * C + c);
-                                } else if constexpr (kMode == 2) {
-                                    static_cast<float*>(a.out)[((int64_t)ub * a.c_total + a.c_offset + c) * ipt + ur + i] = ob;
-                                } else {
-                                    if (f32) rows_dst[(int64_t)i * rs + m * 128] = ob;
-                                    else rows_dst16[(int64_t)i * rs + m * 128] = to_16bit(ob, a.out_dtype);
-                                }
-                            }
-                        }
-                    }
-                }
-                rows_dst += rows_step;
-                rows_dst16 += rows_step;
-            }
-        }
     } else {
         // =========================== epilogue: group g owns channel tile g ===========================
-        if constexpr (kRegEpi < 80) setmaxnreg_dec<kRegEpi>();
-        if constexpr (kRegEpi > 80) setmaxnreg_inc<kRegEpi>();
+        setmaxnreg_dec<kRegEpi>();
         const int g = (warp - kEpiWarp0) >> 2;
         const int quad = warp & 3;  // TMEM lanes this warp may read: 32 * (warp id % 4)
         const bool nchw = (kMode == 2) || (kMode == 0 && canvas && (a.out_layout == P3P_LAYOUT_NCHW));
@@ -1079,15 +939,13 @@ __global__ void __launch_bounds__(kThreadsOf<kMode>, 1) pfn_tc_kernel(PfnArgs a)
         const uint32_t tf_sa = opaque(smem_u32(t_full + g * kAccStages));   // stage s: + 8 s
         const uint32_t te_sa = opaque(smem_u32(t_empty + g * kAccStages));
         const uint32_t gtf_sa = opaque(smem_u32(gt_full + 2 * g)), gte_sa = opaque(smem_u32(gt_empty + 2 * g));  // slot: + 8
-        const int my_pillars = (g < MT) ? my_units * kUnit : 0;
         int jn = 0;
         // Pillar q of the CTA sits in accumulator stage q & 1 of the tile; its barrier phase is (q >> 1) & 1.  The probe of
         // the NEXT pillar's barrier is issued before the arithmetic on the current one, so that in the steady state (the
         // issuer runs ahead) no wait is exposed.
         uint32_t ready = 0;
-        bool inflight = false;  // the first 16 columns of the pillar in work are already on their way into va
         float va[16], vb[16];
-        const uint32_t rmax_sa = opaque(smem_u32(sRmax + (warp - kEpiWarp0) * (2 * kUnit * 32) + lane));  // [2][kUnit][32 lanes] strips of this warp
+        const uint32_t rmax_sa = opaque(smem_u32(sRmax + (warp - kEpiWarp0) * (kUnit * 32) + lane));  // [kUnit][32 lanes] strip of this warp (thread-private words)
         const uint32_t valid_sa = opaque(smem_u32(sValid));
         const uint32_t taddr_o = opaque(taddr);
         // rows layout: this thread's channel of the unit's first cell; advanced by one pointer addition per unit
@@ -1100,7 +958,7 @@ __global__ void __launch_bounds__(kThreadsOf<kMode>, 1) pfn_tc_kernel(PfnArgs a)
         auto unit_tail = [&](int j, int ub, int ur, int item0) {
             float rmax[kUnit];
 #pragma unroll
-            for (int i = 0; i < kUnit; ++i) rmax[i] = lds_f32(rmax_sa + (uint32_t)((j & 1) * (kUnit * 128) + i * 128));
+            for (int i = 0; i < kUnit; ++i) rmax[i] = lds_f32(rmax_sa + (uint32_t)(i * 128));
             // ---- W1b' hmax of the unit's 8 items (one MMA per unit), bias, relu, the 8 cells ---------------------------
             float gv[8];
             mbar_wait_sa(gtf_sa + 8u * ((uint32_t)j & 1u), ((uint32_t)j >> 1) & 1u);
@@ -1196,7 +1054,6 @@ __global__ void __launch_bounds__(kThreadsOf<kMode>, 1) pfn_tc_kernel(PfnArgs a)
             rows_dst16 += rows_step;
             if (quad == 0) PTL(9 + g, 8 * j + 7, 3);
         };
-        int prev_ub = 0, prev_ur = 0, prev_item0 = 0;
         const int my_units_g = (g < MT) ? my_units : 0;
         for (int j = 0; j < my_units_g; ++j) {
             const int ub = wu.b, ur = wu.r;  // tile / position of the unit's first item
@@ -1204,38 +1061,24 @@ __global__ void __launch_bounds__(kThreadsOf<kMode>, 1) pfn_tc_kernel(PfnArgs a)
             wu.step();
             unit_item0 += ((int)gridDim.x * kUnit) >> bs;
             // ---- the unit's 8 pillars: max over each pillar's 64 accumulator columns ---------------------------------
-            // (a rolled loop over the pairs: the register blocks of the loads keep one assignment; the pillar maxima wait
-            // for the unit's W1b' hmax term in a per-warp shared-memory strip, not in registers).  Four loads of 16
-            // columns per pillar through two register buffers: the arithmetic on one buffer overlaps the load into the
-            // other.
-#if P3P_EPI_UNROLL
+            // (the loop over the pairs is unrolled: barrier parities, strip offsets and probe conditions become constants of
+            // the body; the pillar maxima wait for the unit's W1b' hmax term in a per-warp shared-memory strip, not in
+            // registers).  Four loads of 16 columns per pillar through two register buffers: the arithmetic on one buffer
+            // overlaps the load into the other.
 #pragma unroll
-#else
-#pragma unroll 1
-#endif
             for (int pr = 0; pr < kPairsPerUnit; ++pr) {
 #pragma unroll
                 for (int s = 0; s < kAccStages; ++s, ++jn) {
-#if P3P_EPI_UNROLL
                     const uint32_t tph = (uint32_t)pr & 1u;  // jn = 8 j + 2 pr + s: (jn >> 1) & 1 is a constant of the unrolled body
-#else
-                    const uint32_t tph = (uint32_t)(jn >> 1) & 1u;
-#endif
                     if (quad == 0) PTL(9 + g, jn, 0);
-                    if (!inflight) {
-                        if (!ready) mbar_wait_sa(tf_sa + 8u * s, tph);
-                        tc_fence_after();
-                        tmem_ld16_issue(taddr_o + (uint32_t)(s * kAccCols), va);
-                    }
+                    if (!ready) mbar_wait_sa(tf_sa + 8u * s, tph);
+                    tc_fence_after();
+                    tmem_ld16_issue(taddr_o + (uint32_t)(s * kAccCols), va);
                     if (quad == 0) PTL(9 + g, jn, 1);
                     tmem_ld_wait16(va);
                     tmem_ld16_issue(taddr_o + (uint32_t)(s * kAccCols + 16), vb);
-#if P3P_EPI_UNROLL
                     // (inside a unit the next pillar always exists; behind its last pillar only if another unit follows)
                     ready = (2 * pr + s + 1 < kUnit || j + 1 < my_units_g) ? mbar_test_sa(tf_sa + 8u * (s ^ 1), (uint32_t)((2 * pr + s + 1) >> 1) & 1u) : 0u;
-#else
-                    ready = (jn + 1 < my_pillars) ? mbar_test_sa(tf_sa + 8u * (s ^ 1), (uint32_t)((jn + 1) >> 1) & 1u) : 0u;
-#endif
                     const float r0 = max16(va);
                     tmem_ld_wait16(vb);
                     tmem_ld16_issue(taddr_o + (uint32_t)(s * kAccCols + 32), va);
@@ -1246,31 +1089,12 @@ __global__ void __launch_bounds__(kThreadsOf<kMode>, 1) pfn_tc_kernel(PfnArgs a)
                     tmem_ld_wait16(vb);
                     tc_fence_before();
                     mbar_arrive_sa(te_sa + 8u * s);
-                    // (the vote makes the decision warp-uniform: tcgen05.ld is a warp-wide instruction)
-#if P3P_EPI_PIPE
-                    inflight = __all_sync(0xffffffffu, ready != 0u) != 0;
-                    ready = inflight ? 1u : 0u;
-                    if (inflight) {
-                        tc_fence_after();
-                        tmem_ld16_issue(taddr_o + (uint32_t)((s ^ 1) * kAccCols), va);
-                    }
-#endif
-                    sts_f32(rmax_sa + (uint32_t)((j & 1) * (kUnit * 128) + (2 * pr + s) * 128), max16_with(r2, vb));
+                    sts_f32(rmax_sa + (uint32_t)((2 * pr + s) * 128), max16_with(r2, vb));
                     if (quad == 0) PTL(9 + g, jn, 2);
                 }
-                // (P3P_EPI_DEFER: the PREVIOUS unit's tail runs here, after this unit's first pair)
-#if P3P_EPI_DEFER
-                if (pr == 0 && j > 0) unit_tail(j - 1, prev_ub, prev_ur, prev_item0);
-#endif
             }
-#if !P3P_EPI_DEFER
             unit_tail(j, ub, ur, item0);
-#endif
-            prev_ub = ub; prev_ur = ur; prev_item0 = item0;
         }
-#if P3P_EPI_DEFER
-        if (my_units_g > 0) unit_tail(my_units_g - 1, prev_ub, prev_ur, prev_item0);
-#endif
     }
     tc_fence_before();
     __syncthreads();
@@ -1349,7 +1173,6 @@ int launch_pfn_tc(const PfnArgs& a_in, int precision, cudaStream_t st) {
     cfg.numAttrs = 1;
 #define P3P_LAUNCH_TC(PREC, MODE)                      \
     do {                                               \
-        cfg.blockDim = dim3(kThreadsOf<MODE>);         \
         cfg.dynamicSmemBytes = TcCfg<PREC>::kSmemBytes; \
         P3P_CUDA_CHECK(cudaFuncSetAttribute(pfn_tc_kernel<PREC, MODE>, cudaFuncAttributeMaxDynamicSharedMemorySize, \
                                             (int)TcCfg<PREC>::kSmemBytes)); /* per device context: set per launch */ \

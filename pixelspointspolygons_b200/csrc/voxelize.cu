@@ -303,10 +303,7 @@ constexpr unsigned kKeyMask = (1u << kKeyBits) - 1u;
 static_assert(kMaxKeys <= (1 << kKeyBits), "key field too narrow");
 static_assert(kMaxChunkPoints * 8 < 65536, "8 chunk rows must add up inside 16-bit lanes");
 constexpr int kGroups = kIters / 4;        // groups of 4 consecutive points (48 bytes = 3 x 16-byte loads) per thread
-#ifndef P3P_CROSS_BATCH
-#define P3P_CROSS_BATCH 256
-#endif
-constexpr int kCrossBatch = P3P_CROSS_BATCH;  // crossing keys resolved per round (512 measured: slower, the larger scratch costs L1)
+constexpr int kCrossBatch = 256;           // crossing keys resolved per round (512 measured: no change)
 constexpr int kCells = kGroups * kWarps;   // the chunk-local order is (group, warp, lane, e): 32 cells (group, warp) of 128 consecutive points
 static_assert(kMaxChunkPoints / kCells <= 255, "points of a cell must fit the 8-bit fields of the boundary word");
 constexpr unsigned kCrossFlag = 0x8000u;   // base_s entry: the key crosses M inside this chunk; low 15 bits = crossing id
