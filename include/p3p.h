@@ -234,6 +234,20 @@ int p3p_patch_embed_prepared(const float* images, int32_t num_tiles, int32_t in_
                              void* stream);
 
 /*
+ * The same convolution on the decoded image as a loader holds it before its normalisation: images (B, H, W, in_chans)
+ * uint8, channels-last, 8-byte aligned, in_chans 1..4; pixel_lut (in_chans, 256) fp32 on the device, pixel_lut[c][u] the
+ * value the loader's normalisation gives byte u of channel c (torchvision ToTensor: u / 255).  The result equals
+ * p3p_patch_embed / p3p_patch_embed_prepared on the fp32 image (B, in_chans, H, W) with x[b][c][y][x] =
+ * pixel_lut[c][images[b][y][x][c]], bit for bit: the same route, the same row group, the same operand rounding.  blob:
+ * prepared weights (as for p3p_patch_embed_prepared) or NULL (then weight is required); the table is read by every call
+ * (a CUDA graph that captured one sees later in-place updates of it).
+ */
+int p3p_patch_embed_u8(const uint8_t* images, const float* pixel_lut, int32_t num_tiles, int32_t in_chans, int32_t height,
+                       int32_t width, int32_t patch, const void* blob, const float* weight, const float* bias, int32_t channels,
+                       int32_t precision, void* out, int32_t out_dtype, int32_t out_layout, int32_t c_total, int32_t c_offset,
+                       void* stream);
+
+/*
  * LiDAR input front end (SURVEY 8a row a1 / 8f-3): raw LAS integer coordinates of a jagged batch -> the (total_points, 3)
  * fp32 pixel-space points p3p_encode consumes, bit-identical to the numpy / scikit-learn code of
  * P3Dataset.load_lidar_points (p3_coco.py:74-101; clip = 1) and Predictor.load_lidar_from_file (predictor.py:116-137;

@@ -17,7 +17,7 @@ EXPORTED = [
     "p3p_voxelize", "p3p_pillar_features", "p3p_encode", "p3p_encode_tokens", "p3p_patch_embed", "p3p_las_to_pixels",
     "p3p_profile_begin", "p3p_profile_end", "p3p_conv3x3_blob_bytes", "p3p_conv3x3_prepare", "p3p_conv3x3", "p3p_conv3x3_vit_tokens",
     "p3p_nchw_to_nhwc16", "p3p_upsample_bilinear_nhwc16", "p3p_las_packed_to_pixels",
-    "p3p_patch_embed_blob_bytes", "p3p_patch_embed_prepare", "p3p_patch_embed_prepared",
+    "p3p_patch_embed_blob_bytes", "p3p_patch_embed_prepare", "p3p_patch_embed_prepared", "p3p_patch_embed_u8",
     "p3p_encode_workspace", "p3p_pfn_train_state_doubles", "p3p_pfn_train_route_bytes", "p3p_pfn_train_stats0",
     "p3p_pfn_train_stats1", "p3p_pfn_train_stats2", "p3p_pfn_train_forward", "p3p_pfn_backward1", "p3p_pfn_backward2", "p3p_pfn_backward3",
 ]
@@ -105,6 +105,8 @@ def lib():
     l.p3p_patch_embed_prepare.argtypes = [vp, vp, i32, i32, i32, i32, vp, sz, vp]
     l.p3p_patch_embed_prepared.restype = C.c_int
     l.p3p_patch_embed_prepared.argtypes = [vp, i32, i32, i32, i32, i32, vp, vp, vp, i32, i32, vp, i32, i32, i32, i32, vp]
+    l.p3p_patch_embed_u8.restype = C.c_int
+    l.p3p_patch_embed_u8.argtypes = [vp, vp, i32, i32, i32, i32, i32, vp, vp, vp, i32, i32, vp, i32, i32, i32, i32, vp]
     l.p3p_conv3x3_blob_bytes.restype = sz
     l.p3p_conv3x3_blob_bytes.argtypes = [i32, i32]
     l.p3p_conv3x3_prepare.restype = C.c_int

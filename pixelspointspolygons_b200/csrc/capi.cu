@@ -580,4 +580,25 @@ int p3p_patch_embed_prepared(const float* images, int32_t num_tiles, int32_t in_
                               out_layout, c_total, c_offset, static_cast<cudaStream_t>(stream));
 }
 
+int p3p_patch_embed_u8(const uint8_t* images, const float* pixel_lut, int32_t num_tiles, int32_t in_chans, int32_t height,
+                       int32_t width, int32_t patch, const void* blob, const float* weight, const float* bias, int32_t channels,
+                       int32_t precision, void* out, int32_t out_dtype, int32_t out_layout, int32_t c_total, int32_t c_offset,
+                       void* stream) {
+    if (!pixel_lut) return fail(P3P_ERR_INVALID_ARGUMENT, "null pixel_lut");
+    if (in_chans < 1 || in_chans > 4) return fail(P3P_ERR_UNSUPPORTED, "in_chans %d of a uint8 image (supported: 1..4)", in_chans);
+    const int rc = p3p_patch_embed(nullptr, 0, in_chans, height, width, patch, weight, bias, channels, precision, out, out_dtype,
+                                   out_layout, c_total, c_offset, stream);  // (argument checks; no tiles: no launch)
+    if (rc) return rc;
+    if (num_tiles < 0) return fail(P3P_ERR_INVALID_ARGUMENT, "num_tiles %d", num_tiles);
+    if (num_tiles == 0) return P3P_OK;
+    if (!images || !out) return fail(P3P_ERR_INVALID_ARGUMENT, "null images or out");
+    if (!blob && !weight) return fail(P3P_ERR_INVALID_ARGUMENT, "null weight and blob");
+    if (reinterpret_cast<uintptr_t>(images) & 7u) return fail(P3P_ERR_INVALID_ARGUMENT, "images must be 8-byte aligned");
+    if (!aligned16(out) || (weight && !aligned16(weight)) || (blob && !aligned16(blob)) || (reinterpret_cast<uintptr_t>(pixel_lut) & 3u))
+        return fail(P3P_ERR_INVALID_ARGUMENT, "misaligned pointer");
+    return launch_patch_embed(nullptr, num_tiles, in_chans, height, width, patch, weight, bias,
+                              (patch == 8 && precision != P3P_PRECISION_FP32) ? blob : nullptr, channels, precision, out, out_dtype,
+                              out_layout, c_total, c_offset, static_cast<cudaStream_t>(stream), images, pixel_lut);
+}
+
 }  // extern "C"

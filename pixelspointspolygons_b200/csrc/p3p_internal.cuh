@@ -180,7 +180,7 @@ size_t patch_embed_blob_bytes(int C, int in_chans, int P);
 int launch_patch_embed_prepare(const float* weight, const float* bias, int C, int in_chans, int P, int precision, void* blob, cudaStream_t st);
 int launch_patch_embed(const float* images, int B, int in_chans, int H, int W, int P, const float* weight, const float* bias,
                        const void* blob, int C, int precision, void* out, int out_dtype, int out_layout, int c_total, int c_offset,
-                       cudaStream_t st);
+                       cudaStream_t st, const uint8_t* images_u8 = nullptr, const float* pixel_lut = nullptr);
 int launch_las_to_pixels(const int32_t* X, const int32_t* Y, const int32_t* Z, const uint16_t* deltas, const int32_t* base,
                          const int64_t* offsets, int B, int64_t total, const p3p_las_tile* tiles, double z_hi, int32_t* mm, float* out,
                          cudaStream_t st);

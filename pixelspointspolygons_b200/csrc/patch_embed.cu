@@ -16,10 +16,21 @@
 //   TMEM; tcgen05.mma kind::tf32 (fp32 contract) or kind::f16 on bf16 operands (bf16 contract), fp32 accumulate;
 //   epilogue: tcgen05.ld, + bias, NCHW rows of R*nx contiguous values per channel.
 // patch_embed_simt_kernel: exact fp32 FMA for any P / shape -- the GPU-side cross-check and the fp32 route.
+//
+// Both kernels take the image in one of two formats, a compile-time parameter (kIn):
+//   kInF32:  (B, in_chans, H, W) fp32 NCHW, already normalised by the loader;
+//   kInU8:   (B, H, W, in_chans) uint8 channels-last -- the decoded image as the loader holds it before its Normalize /
+//            ToTensor -- with a pixel table lut (in_chans, 256) fp32: pixel value = lut[c][byte].  Every per-channel pointwise
+//            normalisation is such a table, so the conversion is exact whatever arithmetic the loader used.  The table is
+//            copied to a static shared array (4 KB), outside the dynamic shared-memory budget: both formats take the same
+//            route with the same row group, and the u8 image moves a quarter of the fp32 bytes.
 #include "p3p_internal.cuh"
 
 namespace p3p {
 namespace {
+
+constexpr int kInF32 = 0, kInU8 = 1;  // image formats (see the file comment)
+constexpr int kMaxU8Chans = 4;      // channels of a u8 image: one 8-byte load per channel per 8-pixel span
 
 __device__ __forceinline__ void store_out(void* out, int out_dtype, int64_t idx, float v) {
     if (out_dtype == P3P_DTYPE_F32)
@@ -31,9 +42,12 @@ __device__ __forceinline__ void store_out(void* out, int out_dtype, int64_t idx,
 // ------------------------------------------------------------------------------------------------
 // exact fp32 kernel: one CTA per (cell, image); the patch sits in shared memory, one thread per channel
 // ------------------------------------------------------------------------------------------------
+// kInU8: img is NULL; img8 (B, H, W, in_chans) and lut (in_chans, 256) are read instead
+template <int kIn>
 __global__ void __launch_bounds__(128)
 patch_embed_simt_kernel(const float* __restrict__ img, int in_chans, int H, int W, int P, const float* __restrict__ weight,
-                        const float* __restrict__ bias, int C, void* out, int out_dtype, int out_layout, int c_total, int c_offset) {
+                        const float* __restrict__ bias, int C, void* out, int out_dtype, int out_layout, int c_total, int c_offset,
+                        const unsigned char* __restrict__ img8, const float* __restrict__ lut) {
     extern __shared__ float patch[];  // [in_chans * P * P]
     const int nx = W / P, ny = H / P;
     const int cell = blockIdx.x, b = blockIdx.y;
@@ -41,7 +55,10 @@ patch_embed_simt_kernel(const float* __restrict__ img, int in_chans, int H, int 
     const int K = in_chans * P * P;
     for (int k = threadIdx.x; k < K; k += blockDim.x) {
         const int c = k / (P * P), r = k - c * P * P, py = r / P, px = r - py * P;
-        patch[k] = img[(((int64_t)b * in_chans + c) * H + cy * P + py) * W + cx * P + px];
+        if constexpr (kIn == kInU8)
+            patch[k] = __ldg(lut + c * 256 + img8[(((int64_t)b * H + cy * P + py) * W + cx * P + px) * in_chans + c]);
+        else
+            patch[k] = img[(((int64_t)b * in_chans + c) * H + cy * P + py) * W + cx * P + px];
     }
     __syncthreads();
     for (int ch = threadIdx.x; ch < C; ch += blockDim.x) {
@@ -70,6 +87,8 @@ struct PeArgs {
     int rows;       // cell rows per CTA
     int N;          // rows * nx: MMA N (multiple of 16, <= 128)
     int out_dtype, out_layout, c_total, c_offset;
+    const unsigned char* img8;  // kInU8: (B, H, W, in_chans) uint8 (img is NULL) ...
+    const float* lut;           // ... and its pixel table (in_chans, 256)
 };
 
 // Operand rows are K-major and split into 128-byte chunks (SWIZZLE_128B atoms, 8 rows x 128 B); chunk q of a tile
@@ -101,12 +120,32 @@ __device__ __forceinline__ void put_run(unsigned char* tile, int nrows, int row,
     }
 }
 
+// One span of a u8 image: 8 pixels x kIC bytes (pixel-major, as the image stores them) of pixel row py of a cell, loaded as
+// kIC 8-byte words.  Byte c of every pixel goes through the channel's table to the fp32 run (c, py), which put_run converts
+// and stores exactly as it does an fp32 image's run.  (kIC is a template parameter so that every byte position is a constant:
+// the bytes are picked out of registers, no local-memory array.)
+template <int kPrec, int kIC>
+__device__ __forceinline__ void put_span_u8(unsigned char* tile, int nrows, int row, int py, const uint2 (&w)[kMaxU8Chans],
+                                            const float* lut) {
+#pragma unroll
+    for (int c = 0; c < kIC; ++c) {
+        float v[8];
+#pragma unroll
+        for (int p = 0; p < 8; ++p) {
+            const int j = p * kIC + c;  // byte of the span
+            const uint32_t word = (j & 4) ? w[j >> 3].y : w[j >> 3].x;
+            v[p] = lut[c * 256 + ((word >> ((j & 3) * 8)) & 0xffu)];
+        }
+        put_run<kPrec>(tile, nrows, row, c * 8 + py, make_float4(v[0], v[1], v[2], v[3]), make_float4(v[4], v[5], v[6], v[7]));
+    }
+}
+
 // CTA = (row group of R cell rows, image): the B operand (the pixel runs of the row group, the only HBM read) is built ONCE
 // and multiplied with every 128-channel tile of the weights -- kTilesResident tiles at a time (all three of C = 384 with
 // 16-bit operands; one with tf32, whose tiles are twice as large), each tile an MMA chain into its own TMEM columns with its
 // own commit barrier, so that the epilogue of tile m runs under the MMAs of tile m + 1.  (r01: one CTA per (row group,
 // channel tile, image) re-read the image slab three times and idled through load -> MMA -> epilogue; 28 us at B = 16.)
-template <int kPrec>
+template <int kPrec, int kIn>
 __global__ void __launch_bounds__(kPeThreads, 1) patch_embed_tc_kernel(PeArgs a) {
     constexpr bool kTf32 = (kPrec == P3P_PRECISION_TF32);
     constexpr int kTilesResident = kTf32 ? 1 : 3;
@@ -135,7 +174,15 @@ __global__ void __launch_bounds__(kPeThreads, 1) patch_embed_tc_kernel(PeArgs a)
         fence_mbar_init();
     }
     const bool prepared = a.blob != nullptr;
-    if (prepared) __syncthreads();  // (the barrier is initialised before the copies that complete on it are issued)
+    float* lut_s = nullptr;  // kInU8: the pixel table in static shared memory (not in the dynamic operand budget)
+    if constexpr (kIn == kInU8) {
+        __shared__ float lut_tab[kMaxU8Chans * 256];
+        lut_s = lut_tab;
+        for (int i = tid; i < a.in_chans * 256; i += kPeThreads) lut_s[i] = __ldg(a.lut + i);
+    }
+    // (the barrier is initialised before the copies that complete on it are issued; the table is in place before the
+    // pixel spans are built)
+    if (kIn == kInU8 || prepared) __syncthreads();
     // 32-byte runs -> operand rows.  A: 128 channels x K weights of tile mt, natural (C, in_chans, 8, 8) order == K-major
     // rows; B: the pixel runs of `rows` cell rows: image rows (c, cy0*8 + y), nx runs each.  kDepth runs (2 x float4 each) per
     // thread in flight.
@@ -184,6 +231,40 @@ __global__ void __launch_bounds__(kPeThreads, 1) patch_embed_tc_kernel(PeArgs a)
             }
         }
     };
+    // u8 image: the B operand from the spans of `rows` cell rows -- image rows cy0*8 + y, nx spans of 8 pixels x in_chans
+    // bytes each, consecutive threads on consecutive spans of a row (coalesced), kDepthU8 spans per thread in flight
+    auto load_spans_u8 = [&]() {
+        if constexpr (kIn == kInU8) {
+            constexpr int kDepthU8 = 4;
+            const int spans = a.rows * 8 * a.nx;
+            const int span_bytes = 8 * a.in_chans;
+            const unsigned char* src8 = a.img8 + ((size_t)b * a.H + (size_t)cy0 * 8) * a.W * a.in_chans;
+            for (int i0 = tid; i0 < spans; i0 += kPeThreads * kDepthU8) {
+                uint2 w[kDepthU8][kMaxU8Chans];
+#pragma unroll
+                for (int d = 0; d < kDepthU8; ++d) {
+                    const int i = i0 + d * kPeThreads;
+                    const int yl = i / a.nx, cx = i - yl * a.nx;
+                    const uint2* src = reinterpret_cast<const uint2*>(src8 + (size_t)yl * a.W * a.in_chans + (size_t)cx * span_bytes);
+#pragma unroll
+                    for (int c = 0; c < kMaxU8Chans; ++c) w[d][c] = (i < spans && c < a.in_chans) ? __ldg(src + c) : make_uint2(0u, 0u);
+                }
+#pragma unroll
+                for (int d = 0; d < kDepthU8; ++d) {
+                    const int i = i0 + d * kPeThreads;
+                    if (i >= spans) break;
+                    const int yl = i / a.nx, cx = i - yl * a.nx;
+                    const int row = (yl >> 3) * a.nx + cx, py = yl & 7;
+                    switch (a.in_chans) {
+                        case 1: put_span_u8<kPrec, 1>(sB, Npad, row, py, w[d], lut_s); break;
+                        case 2: put_span_u8<kPrec, 2>(sB, Npad, row, py, w[d], lut_s); break;
+                        case 3: put_span_u8<kPrec, 3>(sB, Npad, row, py, w[d], lut_s); break;
+                        default: put_span_u8<kPrec, 4>(sB, Npad, row, py, w[d], lut_s); break;
+                    }
+                }
+            }
+        }
+    };
     const int quad = warp & 3, hi_half = warp >> 2;
     // The fp32 NCHW epilogue stages its transposes in a weight tile's space, 8 warps x 32 x 17 floats.  A 16-bit tile of one
     // input channel is 16 KB, smaller than that: past its end lie the next tile, still under its MMAs, or the image operand,
@@ -209,9 +290,16 @@ __global__ void __launch_bounds__(kPeThreads, 1) patch_embed_tc_kernel(PeArgs a)
                     asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(smem_u32(sA + (size_t)t * a_tile_bytes)),
                                  "l"(a.blob + (size_t)(mt0 + t) * a_tile_bytes), "r"((uint32_t)a_tile_bytes), "r"(smem_u32(&abar)) : "memory");
             }
-            load_runs(mt0, 0, mt0 == 0);
+            if constexpr (kIn == kInU8) {
+                if (mt0 == 0) load_spans_u8();
+            } else {
+                load_runs(mt0, 0, mt0 == 0);
+            }
         } else {
-            load_runs(mt0, ntiles, mt0 == 0);
+            load_runs(mt0, ntiles, kIn == kInF32 && mt0 == 0);
+            if constexpr (kIn == kInU8) {
+                if (mt0 == 0) load_spans_u8();
+            }
         }
         fence_async_smem();
         tc_fence_before();
@@ -339,11 +427,14 @@ int launch_patch_embed_prepare(const float* weight, const float* bias, int C, in
     return P3P_OK;
 }
 
-// blob: the prepared weights of `precision` (p3p_patch_embed_prepare) or NULL (raw weights converted by every CTA)
+// blob: the prepared weights of `precision` (p3p_patch_embed_prepare) or NULL (raw weights converted by every CTA).
+// images_u8 (B, H, W, in_chans) uint8 + pixel_lut (in_chans, 256), when given, replace the fp32 NCHW images; the route and
+// the row group do not depend on the image format.
 int launch_patch_embed(const float* images, int B, int in_chans, int H, int W, int P, const float* weight, const float* bias,
                        const void* blob, int C, int precision, void* out, int out_dtype, int out_layout, int c_total, int c_offset,
-                       cudaStream_t st) {
+                       cudaStream_t st, const uint8_t* images_u8, const float* pixel_lut) {
     if (B <= 0) return P3P_OK;
+    const bool u8 = images_u8 != nullptr;
     const int nx = W / P, ny = H / P;
     const bool tf32 = (precision != P3P_PRECISION_BF16 && precision != P3P_PRECISION_FP16);
     // tensor-core route: 8x8 patches; a row group of `rows` cell rows with rows * nx a multiple of 16 and <= 128 that
@@ -360,12 +451,9 @@ int launch_patch_embed(const float* images, int B, int in_chans, int H, int W, i
     const size_t smem = 1024 + ((tf32 ? 1 : 3) * 128 + (size_t)rows * nx) * K * esize;  // resident weight tiles + the row group
     const bool k_ok = tf32 ? (K % 32 == 0) : (K % 64 == 0);
     if (rows > 0 && k_ok && smem <= 200 * 1024 && ((size_t)ny * nx * (out_dtype == P3P_DTYPE_F32 ? 4 : 2)) % 16 == 0) {
-        // (the attribute belongs to the current device's context: set per launch, it is cheap)
-        P3P_CUDA_CHECK(cudaFuncSetAttribute(patch_embed_tc_kernel<P3P_PRECISION_TF32>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
-        P3P_CUDA_CHECK(cudaFuncSetAttribute(patch_embed_tc_kernel<P3P_PRECISION_BF16>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
-        P3P_CUDA_CHECK(cudaFuncSetAttribute(patch_embed_tc_kernel<P3P_PRECISION_FP16>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
         PeArgs a;
         a.img = images; a.weight = weight; a.bias = bias; a.out = out;
+        a.img8 = images_u8; a.lut = pixel_lut;
         a.blob = static_cast<const unsigned char*>(blob);
         if (blob)  // the bias (padded to whole tiles, zeros without one) follows the tiles
             a.bias = reinterpret_cast<const float*>(a.blob + (size_t)((C + 127) / 128) * 128 * K * esize);
@@ -373,20 +461,29 @@ int launch_patch_embed(const float* images, int B, int in_chans, int H, int W, i
         a.rows = rows; a.N = rows * nx;
         a.out_dtype = out_dtype; a.out_layout = out_layout; a.c_total = c_total; a.c_offset = c_offset;
         dim3 grid((unsigned)(ny / rows), (unsigned)B);
+        // (the attribute belongs to the current device's context: set per launch, it is cheap)
+        auto launch = [&](auto kernel) -> int {
+            P3P_CUDA_CHECK(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
+            kernel<<<grid, kPeThreads, smem, st>>>(a);
+            P3P_CUDA_CHECK(cudaGetLastError());
+            return P3P_OK;
+        };
         if (tf32)
-            patch_embed_tc_kernel<P3P_PRECISION_TF32><<<grid, kPeThreads, smem, st>>>(a);
-        else if (precision == P3P_PRECISION_BF16)
-            patch_embed_tc_kernel<P3P_PRECISION_BF16><<<grid, kPeThreads, smem, st>>>(a);
-        else
-            patch_embed_tc_kernel<P3P_PRECISION_FP16><<<grid, kPeThreads, smem, st>>>(a);
-        P3P_CUDA_CHECK(cudaGetLastError());
-        return P3P_OK;
+            return u8 ? launch(patch_embed_tc_kernel<P3P_PRECISION_TF32, kInU8>) : launch(patch_embed_tc_kernel<P3P_PRECISION_TF32, kInF32>);
+        if (precision == P3P_PRECISION_BF16)
+            return u8 ? launch(patch_embed_tc_kernel<P3P_PRECISION_BF16, kInU8>) : launch(patch_embed_tc_kernel<P3P_PRECISION_BF16, kInF32>);
+        return u8 ? launch(patch_embed_tc_kernel<P3P_PRECISION_FP16, kInU8>) : launch(patch_embed_tc_kernel<P3P_PRECISION_FP16, kInF32>);
     }
     if (!weight) return fail(P3P_ERR_UNSUPPORTED, "this shape / precision takes the exact route, which needs the raw weights");
     const size_t smem_simt = (size_t)in_chans * P * P * sizeof(float);
     if (smem_simt > 48 * 1024) return fail(P3P_ERR_UNSUPPORTED, "patch of %d x %d x %d values exceeds the shared-memory budget", in_chans, P, P);
     dim3 grid((unsigned)(ny * nx), (unsigned)B);
-    patch_embed_simt_kernel<<<grid, 128, smem_simt, st>>>(images, in_chans, H, W, P, weight, bias, C, out, out_dtype, out_layout, c_total, c_offset);
+    if (u8)
+        patch_embed_simt_kernel<kInU8><<<grid, 128, smem_simt, st>>>(nullptr, in_chans, H, W, P, weight, bias, C, out, out_dtype, out_layout,
+                                                                   c_total, c_offset, images_u8, pixel_lut);
+    else
+        patch_embed_simt_kernel<kInF32><<<grid, 128, smem_simt, st>>>(images, in_chans, H, W, P, weight, bias, C, out, out_dtype, out_layout,
+                                                                    c_total, c_offset, nullptr, nullptr);
     P3P_CUDA_CHECK(cudaGetLastError());
     return P3P_OK;
 }

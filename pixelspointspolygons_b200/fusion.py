@@ -29,8 +29,20 @@ from ._lib import P3P_LAYOUT_NCHW, P3P_LAYOUT_NLC, P3P_PRECISION
 from .encoder import PointPillarsEncoder, _get, _out_dtype_code
 
 
+def default_pixel_lut(in_chans: int = 3) -> torch.Tensor:
+    """(in_chans, 256) fp32: byte u -> u / 255 in every channel, torchvision's `ToTensor` arithmetic -- with the reference's
+    `image_mean 0, std 1` (config/encoder/early_fusion_vit.yaml:48-50) the whole of its normalisation."""
+    return torch.arange(256, dtype=torch.float32).div(255).expand(int(in_chans), 256).contiguous()
+
+
 class PatchEmbed(nn.Module):
-    """timm.layers.PatchEmbed as the reference uses it (`flatten = False`, norm = Identity, NCHW output)."""
+    """timm.layers.PatchEmbed as the reference uses it (`flatten = False`, norm = Identity, NCHW output).
+
+    Besides the fp32 NCHW image (B, in_chans, H, W) the module takes the decoded image as the loader holds it before its
+    normalisation: uint8 channels-last (B, H, W, in_chans), in_chans <= 4.  A pixel table maps every byte to the value the
+    loader's normalisation would give it (`set_pixel_lut`; default `default_pixel_lut`), and the kernel applies it while it
+    builds its operand, so the result is the one of the fp32 image expanded through the table, bit for bit.  The table is
+    neither a parameter nor a buffer (state_dict keys stay timm's); each device keeps one copy, updated in place."""
 
     def __init__(self, img_size=224, patch_size=8, in_chans=3, embed_dim=384, bias=True, precision: str = "fp16"):
         super().__init__()
@@ -40,6 +52,44 @@ class PatchEmbed(nn.Module):
         self.norm = nn.Identity()
         self.precision = precision
         self._blobs = {}  # (device, precision) -> (parameter stamp, prepared weights)
+        self._pixel_lut = default_pixel_lut(self.in_chans)  # host copy of the table
+        self._luts = {}   # device -> (in_chans, 256) fp32 copy the kernels read
+
+    @property
+    def pixel_lut(self) -> torch.Tensor:
+        """The pixel table (in_chans, 256) fp32 of the uint8 route (a copy on the CPU)."""
+        return self._pixel_lut.clone()
+
+    def set_pixel_lut(self, lut) -> None:
+        """Install the table `lut[c][u]` = the value the loader's normalisation gives byte u of channel c: (in_chans, 256),
+        or (256,) for every channel.  Takes effect on the next call; the device copies are updated in place, so CUDA graphs
+        that captured this module (HostPipeline) read the new table too."""
+        t = torch.as_tensor(lut).detach().to(device="cpu", dtype=torch.float32)
+        if t.shape == (256,):
+            t = t.expand(self.in_chans, 256)
+        if t.shape != (self.in_chans, 256):
+            raise ValueError(f"the pixel table must be ({self.in_chans}, 256) or (256,), got {tuple(t.shape)}")
+        self._pixel_lut = t.contiguous().clone()
+        for dev, d in self._luts.items():
+            with torch.cuda.device(dev):
+                d.copy_(self._pixel_lut)
+                torch.cuda.current_stream(dev).synchronize()  # in place before any stream's next kernel reads it
+
+    def _lut(self, device) -> torch.Tensor:
+        d = self._luts.get(device)
+        if d is None:
+            d = self._luts[device] = self._pixel_lut.to(device)
+        return d
+
+    def expand_pixels(self, x: torch.Tensor) -> torch.Tensor:
+        """uint8 (B, H, W, in_chans) -> the fp32 (B, in_chans, H, W) image it stands for: lut[c][x[b, y, x, c]]."""
+        if x.dtype != torch.uint8 or x.dim() != 4 or x.shape[3] != self.in_chans:
+            raise TypeError(f"x_image must be uint8 (B, H, W, {self.in_chans})")
+        lut = self._lut(x.device) if x.is_cuda else self._pixel_lut
+        idx = x.permute(0, 3, 1, 2).long() + 256 * torch.arange(self.in_chans, device=x.device).view(1, -1, 1, 1)
+        # (the gather keeps the index's channels-last strides; a contiguous NCHW tensor, as the loader's ToTensorV2 + collate
+        # give, makes cuDNN pick the same convolution algorithms as for the fp32 image)
+        return lut.reshape(-1)[idx].contiguous()
 
     def _blob(self, device, precision: str) -> torch.Tensor:
         """The weights as tensor-core operand tiles (p3p_patch_embed_prepare), re-made when a parameter changes."""
@@ -60,18 +110,25 @@ class PatchEmbed(nn.Module):
         self._blobs[(device, precision)] = (stamp, blob)
         return blob
 
+    def _image_hw(self, x: torch.Tensor):
+        """(B, H, W) of an fp32 NCHW or a uint8 NHWC image; anything else is a TypeError."""
+        if x.dim() == 4 and x.dtype == torch.float32 and x.shape[1] == self.in_chans:
+            return x.shape[0], x.shape[2], x.shape[3]
+        if x.dim() == 4 and x.dtype == torch.uint8 and x.shape[3] == self.in_chans:
+            return x.shape[0], x.shape[1], x.shape[2]
+        raise TypeError(f"x_image must be float32 (B, {self.in_chans}, H, W) or uint8 (B, H, W, {self.in_chans})")
+
     def forward_into(self, x: torch.Tensor, out: torch.Tensor, c_total: int, c_offset: int, precision: Optional[str] = None,
                      layout: int = P3P_LAYOUT_NCHW):
         """Conv2d(P x P / P) of `x` into channels [c_offset, c_offset + C) of `out`: NCHW (B, c_total, H/P, W/P) or
-        channels-last rows (B, H/P * W/P, c_total); fp32, bf16 or fp16."""
+        channels-last rows (B, H/P * W/P, c_total); fp32, bf16 or fp16.  x: fp32 (B, in_chans, H, W), or uint8
+        (B, H, W, in_chans) mapped through the pixel table."""
         if not x.is_cuda:
             raise RuntimeError("PatchEmbed runs on CUDA only (sm_100a); x_image is on " + str(x.device))
-        if x.dtype != torch.float32 or x.dim() != 4 or x.shape[1] != self.in_chans:
-            raise TypeError(f"x_image must be float32 (B, {self.in_chans}, H, W)")
+        B, H, W = self._image_hw(x)
         x = x.contiguous()
         w = self.proj.weight.detach().contiguous()
         b = self.proj.bias.detach().contiguous() if self.proj.bias is not None else None
-        B, _, H, W = x.shape
         dt = _out_dtype_code(out)
         need = B * (H // self.patch_size) * (W // self.patch_size) * c_total
         if out.device != x.device or not out.is_contiguous() or out.numel() < need:
@@ -81,18 +138,27 @@ class PatchEmbed(nn.Module):
             raise RuntimeError("PatchEmbed parameters must be float32 on the device of x_image")
         with torch.cuda.device(x.device):
             blob = self._blob(x.device, precision)
+            st = torch.cuda.current_stream(x.device).cuda_stream
+            if x.dtype == torch.uint8:
+                rc = _lib.lib().p3p_patch_embed_u8(x.data_ptr(), self._lut(x.device).data_ptr(), B, self.in_chans, H, W,
+                                                   self.patch_size, blob.data_ptr(), w.data_ptr(),
+                                                   b.data_ptr() if b is not None else None, self.embed_dim, P3P_PRECISION[precision],
+                                                   out.data_ptr(), dt, layout, c_total, c_offset, st)
+                _lib.check(rc, "p3p_patch_embed_u8")
+                return out
             rc = _lib.lib().p3p_patch_embed_prepared(x.data_ptr(), B, self.in_chans, H, W, self.patch_size, blob.data_ptr(),
                                                      w.data_ptr(), b.data_ptr() if b is not None else None, self.embed_dim,
-                                                     P3P_PRECISION[precision], out.data_ptr(), dt, layout, c_total, c_offset,
-                                                     torch.cuda.current_stream(x.device).cuda_stream)
+                                                     P3P_PRECISION[precision], out.data_ptr(), dt, layout, c_total, c_offset, st)
         _lib.check(rc, "p3p_patch_embed_prepared")
         return out
 
     def forward(self, x):
         if self.training and torch.is_grad_enabled():
+            if x.dtype == torch.uint8:  # the same table, then the autograd route
+                x = self.expand_pixels(x)
             y = self.proj(x)  # autograd route of the optional training step
         else:
-            B, _, H, W = x.shape
+            B, H, W = self._image_hw(x) if x.dtype == torch.uint8 else (x.shape[0], x.shape[2], x.shape[3])
             y = torch.empty(B, self.embed_dim, H // self.patch_size, W // self.patch_size, dtype=torch.float32, device=x.device)
             self.forward_into(x, y, self.embed_dim, 0)
         if self.flatten:

@@ -5,8 +5,9 @@ The reference feeds the encoder from a DataLoader: laspy decodes a tile, `P3Data
 function builds the jagged batch (R:pixelspointspolygons/datasets/collate_funcs.py:108) and the trainer / predictor moves
 it to the device before `encoder(x_image, x_lidar)`.  `HostPipeline` is that loop for a GPU whose kernels are an order of
 magnitude faster than the PCIe link: the loader writes what the LAS file holds (integer coordinates as uint16 deltas + an
-int32 base per tile, 6 bytes per point; the tile headers; optionally the fp32 image) straight into a pinned staging slot,
-and per batch the host issues
+int32 base per tile, 6 bytes per point; the tile headers; optionally the image, fp32 NCHW or -- `image_dtype=torch.uint8`
+-- the decoded uint8 channels-last pixels, a quarter of the bytes, normalised by the patch embedding's pixel table on the
+device) straight into a pinned staging slot, and per batch the host issues
 
     copy stream     H2D(slot s + 1)          one copy of the slot's whole arena
     compute stream  compute(slot s)          ONE CUDA-graph launch: las_packed_to_pixels -> voxelize -> PFN (-> patch embed,
@@ -45,7 +46,7 @@ class Slot:
         self.base: torch.Tensor = None     # (B, 3) int32
         self.offsets: torch.Tensor = None  # (B + 1) int64
         self.meta: torch.Tensor = None     # (B * sizeof(p3p_las_tile)) uint8: written by set_tiles
-        self.image: Optional[torch.Tensor] = None  # (B, 3, H, W) float32 (fusion workloads)
+        self.image: Optional[torch.Tensor] = None  # fusion workloads: (B, 3, H, W) float32, or (B, H, W, 3) uint8
         self.out: torch.Tensor = None      # device: the module's output for this slot
         self.host_out: Optional[torch.Tensor] = None    # pinned: full copy of `out` (host_result = "full")
         self.host_value: Optional[torch.Tensor] = None  # pinned: reduce(out) (host_result = callable)
@@ -64,6 +65,12 @@ class HostPipeline:
     -- is seen by the next batch computed, a tensor put in their place (a new `nn.Parameter`, `.to()` elsewhere) is not;
     build a new pipeline for that.
 
+    `image_dtype`: torch.float32 (default) stages the image as the normalised fp32 (B, 3, H, W) tensor; torch.uint8 stages
+    the decoded pixels (B, H, W, 3) as the loader holds them before its Normalize / ToTensor, and the patch embedding maps
+    them through `module.image_embed`'s pixel table (`PatchEmbed.set_pixel_lut`).  The graphs read that table where it is
+    in device memory: `set_pixel_lut` updates it in place and is seen by the next batch computed; a table on a module put in
+    its place is not.
+
     Use:
         s = pipe.staging()        # the slot to fill next (blocks only if its previous copy is still in flight)
         s.deltas[...] = ...; s.base[...] = ...; s.offsets[...] = ...; pipe.set_tiles(s, headers); s.image[...] = ...
@@ -74,7 +81,7 @@ class HostPipeline:
 
     def __init__(self, module, B: int, total: int, slots: int = 3, mode: str = "tokens", image_hw: Sequence[int] = (224, 224),
                  host_result=None, z_hi: float = 100.0, variant: str = "dataset", cls_token: Optional[torch.Tensor] = None,
-                 pos_embed: Optional[torch.Tensor] = None):
+                 pos_embed: Optional[torch.Tensor] = None, image_dtype: torch.dtype = torch.float32):
         if slots < 2:
             raise ValueError("at least two slots (one in compute, one in copy)")
         p = next(module.parameters())
@@ -100,6 +107,9 @@ class HostPipeline:
             self._cls, self._pos = cls_token, pos_embed
         elif cls_token is not None or pos_embed is not None:
             raise ValueError("cls_token / pos_embed belong to mode 'vit_tokens'")
+        if image_dtype not in (torch.float32, torch.uint8):
+            raise ValueError("image_dtype must be torch.float32 or torch.uint8")
+        self.image_dtype = image_dtype
         self._full = host_result == "full"
         self._reduce: Optional[Callable] = host_result if callable(host_result) else None
         if host_result is not None and not (self._full or self._reduce):
@@ -110,7 +120,7 @@ class HostPipeline:
         H, W = int(image_hw[0]), int(image_hw[1])
         sizes = [("deltas", self.total * 6), ("base", self.B * 12), ("offsets", (self.B + 1) * 8), ("meta", self.B * tile_bytes)]
         if self.fusion:
-            sizes.append(("image", self.B * 3 * H * W * 4))
+            sizes.append(("image", self.B * 3 * H * W * (4 if image_dtype == torch.float32 else 1)))
         self._off, pos = {}, 0
         for name, nb in sizes:
             self._off[name] = (pos, nb)
@@ -121,9 +131,12 @@ class HostPipeline:
             def v(name, dtype, shape):
                 o, nb = self._off[name]
                 return arena[o:o + nb].view(dtype).view(*shape)
+            image = None
+            if self.fusion:
+                image = v("image", torch.float32, (self.B, 3, H, W)) if image_dtype == torch.float32 else v("image", torch.uint8, (self.B, H, W, 3))
             d = dict(deltas=v("deltas", torch.uint16, (self.total, 3)), base=v("base", torch.int32, (self.B, 3)),
                      offsets=v("offsets", torch.int64, (self.B + 1,)), meta=v("meta", torch.uint8, (self.B * tile_bytes,)),
-                     image=v("image", torch.float32, (self.B, 3, H, W)) if self.fusion else None)
+                     image=image)
             if slot is not None:
                 for k, t in d.items():
                     setattr(slot, k, t)
